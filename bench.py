@@ -72,7 +72,47 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="skip the (untimed) parity leg")
     ap.add_argument("--cpu-sample", type=int, default=0, help="points of the CPU sample (0 = auto, ~20 s)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy "
+                         "(float64; a fixed seeded sample of the points when the whole batch exceeds 64 MB; "
+                         "rank 0 only; every value finite): coefficients [8, k] in the slot order j_I, alpha_I, j_Q, "
+                         "alpha_Q, j_V, alpha_V, rho_Q, rho_V with 0 where the library returned NaN, nan_mask [8, k] "
+                         "(1 there, 0 elsewhere), status [k] (the per-point status bits, absent for --impl reference) "
+                         "and index [k] (the points' positions in the seeded batch).  --impl reference dumps the sample "
+                         "of its last step, whose size follows the host's cores unless --cpu-sample is given")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_outputs(out_dir, values, status=None, positions=None):
+    """--dump-outputs: values [8, n] (and status [n]) of the last timed step as float64 .npy files, with the
+    positions of the dumped points in the batch.  NaN, the library's marker for a coefficient the reference's
+    algorithm does not produce (or that was not requested), is written as 0 in coefficients.npy and as 1 in
+    nan_mask.npy, so that every dumped value is finite and nothing is lost.  Above DUMP_BYTES_MAX the same
+    seeded sample of points is kept on every run, so that two builds can be compared output for output.
+    `positions` are the points' positions in the seeded batch (default: the batch itself, 0 .. n-1)."""
+    values = np.asarray(values, dtype=np.float64)
+    n = values.shape[1]
+    per_point = 8 * (2 * values.shape[0] + 1 + (status is not None))
+    budget = DUMP_BYTES_MAX - 1024   # the .npy headers
+    if n * per_point > budget:
+        index = np.sort(np.random.default_rng(SEED).choice(n, budget // per_point, replace=False))
+    else:
+        index = np.arange(n)
+    os.makedirs(out_dir, exist_ok=True)
+    kept = values[:, index]
+    nan = np.isnan(kept)
+    np.save(os.path.join(out_dir, "coefficients.npy"), np.where(nan, 0.0, kept))
+    np.save(os.path.join(out_dir, "nan_mask.npy"), nan.astype(np.float64))
+    if status is not None:
+        np.save(os.path.join(out_dir, "status.npy"), np.asarray(status)[index].astype(np.float64))
+    positions = np.arange(n) if positions is None else np.asarray(positions)
+    np.save(os.path.join(out_dir, "index.npy"), positions[index].astype(np.float64))
 
 
 WORKLOADS = {
@@ -221,14 +261,21 @@ def host_threads():
         return max(1, os.cpu_count() or 1)
 
 
+def sample_positions(config, first, count):
+    """Positions in the seeded batch of `config` of the CPU sample's points [first, first + count)."""
+    if config == "juettner_sweep":
+        n = WORKLOADS[config][1]
+        return (np.arange(first, first + count) * 2731) % n  # 2731 is coprime to 16384: a permutation
+    return np.arange(first, first + count)
+
+
 def cpu_sample(config, first, count):
     """Points [first, first + count) of the seeded batch of `config` (rank 0's shard; the sampler is
     prefix-stable, so these are the same points whatever the batch size).  The Juettner sweep is a
     fixed grid: there the sample strides through it, so that every sample covers the whole (T, s) range."""
     if config == "juettner_sweep":
         kind, s, theta, params = draw(config, 0)
-        n = len(s)
-        idx = (np.arange(first, first + count) * 2731) % n  # 2731 is coprime to 16384: a permutation
+        idx = sample_positions(config, first, count)
         return kind, s[idx], theta[idx], [np.asarray(p)[idx] for p in params]
     kind, s, theta, params = draw(config, first + count)
     sl = slice(first, first + count)
@@ -236,7 +283,7 @@ def cpu_sample(config, first, count):
 
 
 def cpu_baseline(config, n_sample, kind_label):
-    """The oracle (the reference's algorithm; its own bessel.c) on the host cores: a bounded sample
+    """The oracle (the reference's algorithm; its own bessel.c where at hand) on the host cores: a bounded sample
     of the same seeded batch, in four sub-batches so that the spread is visible."""
     from oracle import oracle as O
 
@@ -264,7 +311,8 @@ def run_reference(args):
     """--impl reference: the reference's CPU algorithm.  rimphony itself cannot be built in
     this image (no Rust toolchain, no GSL), so this is the oracle port: the restated
     symphony.rs / heyvaerts.rs control flow driving the reference's own bessel.c compiled
-    in place (oracle/_ref).  Rank 0 alone runs; other ranks exit 0.  Every step computes a
+    in place (oracle/_ref), or its restatement oracle/leung_bessel.c where that file is not
+    at hand (oracle.bessel_source()).  Rank 0 alone runs; other ranks exit 0.  Every step computes a
     DIFFERENT slice of the seeded batch (per-point cost spans more than 10x), so K steps time
     K x sample distinct points; the per-step spread is reported."""
     rank = int(os.environ.get("RANK", "0"))
@@ -283,10 +331,12 @@ def run_reference(args):
     for k in range(args.steps):
         kind, s, theta, params = cpu_sample(args.config, k * n_sample, n_sample)
         t0 = time.perf_counter()
-        O.batch(kind, s, theta, params, coeff_mask=mask, n_threads=threads)
+        values, _ = O.batch(kind, s, theta, params, coeff_mask=mask, n_threads=threads)
         dt = time.perf_counter() - t0
         t_all += dt
         rates.append(n_sample / dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, values, positions=sample_positions(args.config, (args.steps - 1) * n_sample, n_sample))
     value = args.steps * n_sample / t_all
     spread = {"min": min(rates), "median": float(np.median(rates)), "max": max(rates), "steps": args.steps}
     points = WORKLOADS[args.config][1] if args.config == "juettner_sweep" else args.points
@@ -346,6 +396,8 @@ def run_single_process(args):
     dt = time.perf_counter() - t0
     clocks = sampler.stop()
     launches = R.kernel_launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out.values, out.status)
     value = n * args.steps / dt
     h2d = 8 * n * (2 + sum(1 for p in params if np.ndim(p))) + 8 * n_dev * sum(1 for p in params if not np.ndim(p))
     d2h = 8 * 8 * n + 4 * n
@@ -434,6 +486,9 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     launches = R.kernel_launch_count() - launches0
     ms_dev = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        # d_out / d_status as the last timed step left them (the legs below write their own buffers)
+        dump_outputs(args.dump_outputs, d_out.view(8, n).cpu().numpy(), d_status.cpu().numpy())
 
     # per-kernel device time and work counters of one more (untimed) step, for the roofline
     res = R.compute_all_dimensionless_batch(kind, s, theta, params, device=local_rank, coeff_mask=mask, extras=True)

@@ -4,10 +4,11 @@ Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s ``cpu_baseline``
 ``--impl reference`` legs may import this module.  The product package
 ``rimphony_b200`` never does (``tests/test_no_oracle_in_product.py`` checks).
 
-The shared objects are built by ``oracle/Makefile``:
-``oracle/_ref/libleung_ref.so`` is the reference's own ``leung-bessel/src/bessel.c``
-compiled in place; ``oracle/_build/liboracle.so`` is the restatement of
-``src/symphony.rs`` / ``src/heyvaerts.rs`` / the four distributions.
+``oracle/Makefile`` builds ``oracle/_build/liboracle.so``, the restatement of
+``src/symphony.rs`` / ``src/heyvaerts.rs`` / the four distributions.  It links the
+reference's own ``leung-bessel/src/bessel.c`` (``oracle/_ref/libleung_ref.so``, prebuilt
+or compiled in place from the reference) and, where neither is at hand, ``leung_bessel.c``,
+a C restatement of it; ``bessel_source()`` says which.
 """
 import ctypes
 import os
@@ -17,7 +18,6 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "_build", "liboracle.so")
-REF_PATH = os.path.join(HERE, "_ref", "libleung_ref.so")
 
 POWER_LAW, THERMAL_JUETTNER, PITCHY_PL, PITCHY_KAPPA = 0, 1, 2, 3
 EMISSION, ABSORPTION, FARADAY = 0, 1, 2
@@ -73,8 +73,8 @@ class Stats(ctypes.Structure):
 
 
 def build(force=False):
-    """Run oracle/Makefile (needs /root/reference only if _ref/ is not prebuilt)."""
-    if force or not (os.path.exists(LIB_PATH) and os.path.exists(REF_PATH)):
+    """Run oracle/Makefile unless liboracle.so is already built."""
+    if force or not os.path.exists(LIB_PATH):
         subprocess.check_call(["make", "-C", HERE, "-s"])
     return LIB_PATH
 
@@ -199,6 +199,14 @@ def set_epsrel(symphony=0.0, heyvaerts=0.0):
 
 def num_threads():
     return lib().orc_num_threads()
+
+
+def bessel_source():
+    """"reference" when liboracle.so runs the reference's own bessel.c (oracle/_ref/libleung_ref.so),
+    "restatement" when it runs oracle/leung_bessel.c."""
+    lib()
+    with open("/proc/self/maps") as f:
+        return "reference" if "libleung_ref.so" in f.read() else "restatement"
 
 
 def ref_bessel_j(n, x):

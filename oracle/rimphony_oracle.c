@@ -16,10 +16,11 @@
  *   src/pitchy_kappa.rs:38-62, 90-125  src/thermal_juettner.rs:29-39, 56-64
  *
  * The Bessel functions J_n, J_n' are NOT restated here: they are the
- * reference's own leung-bessel/src/bessel.c, compiled in place from
- * /root/reference into oracle/_ref/ by oracle/Makefile (pkgw_bessel_j,
- * pkgw_bessel_dj).  GSL QAG / deriv_central are restated in gsl_restated.h,
- * Cephes-backed special functions in special.h.
+ * reference's own leung-bessel/src/bessel.c, compiled in place into
+ * oracle/_ref/ by oracle/Makefile (pkgw_bessel_j, pkgw_bessel_dj), or, where
+ * that file is not at hand, its restatement leung_bessel.c.  GSL QAG /
+ * deriv_central are restated in gsl_restated.h, Cephes-backed special
+ * functions in special.h.
  *
  * This file is the checker (tests/, smoke(), bench.py cpu_baseline and
  * --impl reference).  The product (rimphony_b200/) never links or loads it.

@@ -186,13 +186,51 @@ def test_synthetic_batches_are_reproducible_and_sharded():
 def test_bench_reference_arm_line(tmp_path):
     """bench.py --impl reference prints one JSON line with the contract's keys (tiny sample)."""
     import json
-    out = subprocess.check_output([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                                   "--warmup", "0", "--cpu-sample", "4", "--config", "powerlaw"],
+    out = subprocess.check_output([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2",
+                                   "--warmup", "0", "--cpu-sample", "4", "--config", "powerlaw",
+                                   "--dump-outputs", str(tmp_path / "dump")],
                                   env={**os.environ, "OMP_NUM_THREADS": "4"}, timeout=300)
     line = json.loads(out.decode().strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "coefficient-sets/s" and line["value"] > 0
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
     assert line["higher_is_better"] is True and line["dtype"] == "f64"
+    values = np.load(tmp_path / "dump" / "coefficients.npy")
+    nan_mask = np.load(tmp_path / "dump" / "nan_mask.npy")
+    assert values.shape == nan_mask.shape == (8, 4) and values.dtype == nan_mask.dtype == np.float64
+    assert np.isfinite(values).all() and not nan_mask[:6].any() and (values[0] > 0).all()
+    # the last (second) step computed points 4 .. 7 of the seeded batch, and the dump says so
+    index = np.load(tmp_path / "dump" / "index.npy")
+    assert index.tolist() == [4.0, 5.0, 6.0, 7.0]
+    import bench
+    from oracle import oracle as O
+    kind, s, theta, params = R.synthetic_batch("powerlaw", 8, seed=bench.SEED)
+    sel = index.astype(np.int64)
+    want, _ = O.batch(kind, s[sel], theta[sel], [np.asarray(p)[sel] if np.ndim(p) else p for p in params])
+    assert np.array_equal(np.where(nan_mask == 1.0, np.nan, values), want, equal_nan=True)
+
+
+def test_bench_dump_outputs_is_bounded_and_reproducible(tmp_path):
+    """--dump-outputs: a batch above 64 MB is cut to the same seeded sample of points on every run; NaN is written
+    as 0 with its place in nan_mask, so that every dumped value is finite."""
+    import bench
+    n = 600_000   # 8 coefficients + 8 NaN flags + status + index = 144 bytes per point: 86 MB in all
+    values = np.arange(8 * n, dtype=np.float64).reshape(8, n)
+    values[6:, ::3] = np.nan
+    status = np.arange(n, dtype=np.int32) % 7
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), values, status)
+    total = sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a"))
+    assert 60 << 20 < total <= 64 << 20
+    for f in ("coefficients.npy", "nan_mask.npy", "status.npy", "index.npy"):
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float64 and np.array_equal(a, b) and np.isfinite(a).all()
+    idx = np.load(tmp_path / "a" / "index.npy").astype(np.int64)
+    assert (np.diff(idx) > 0).all()
+    nan_mask = np.load(tmp_path / "a" / "nan_mask.npy")
+    assert np.array_equal(nan_mask == 1.0, np.isnan(values[:, idx])) and nan_mask[6:].any()
+    got = np.where(nan_mask == 1.0, np.nan, np.load(tmp_path / "a" / "coefficients.npy"))
+    assert np.array_equal(got, values[:, idx], equal_nan=True)
+    assert np.array_equal(np.load(tmp_path / "a" / "status.npy"), status[idx].astype(np.float64))
 
 
 def test_high_frequency_approximations_known_answers():

@@ -650,6 +650,27 @@ def test_high_harmonic_corner_runs_and_is_finite():
     assert (res.values[0] > 0).all()
 
 
+def test_bench_dumps_what_the_timed_steps_computed(tmp_path):
+    """bench.py --dump-outputs writes the device buffers of the last timed step: the library's own result for the
+    same seeded points, bit for bit, with its NaNs moved into nan_mask so that every dumped value is finite."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n = 2048
+    subprocess.check_call([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1", "--points", str(n),
+                           "--no-parity", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], timeout=600,
+                          stdout=subprocess.DEVNULL)
+    import bench
+    kind, s, theta, params = bench.draw("pitchy_pl", n)
+    want = R.compute_all_dimensionless_batch(kind, s, theta, params)
+    assert np.load(tmp_path / "index.npy").tolist() == list(range(n))
+    values, nan_mask = np.load(tmp_path / "coefficients.npy"), np.load(tmp_path / "nan_mask.npy")
+    assert np.isfinite(values).all() and np.array_equal(nan_mask == 1.0, np.isnan(want.values))
+    assert np.array_equal(np.where(nan_mask == 1.0, np.nan, values), want.values, equal_nan=True)
+    assert np.array_equal(np.load(tmp_path / "status.npy"), want.status.astype(np.float64))
+
+
 def test_graft_entry_smoke():
     import __graft_entry__ as g
     g.smoke()

@@ -193,6 +193,23 @@ def test_live_oracle_reproduces_fixture(oracle, golden):
     assert np.allclose(lobes, fx["lobes"][:, rows], rtol=1e-12, atol=0.0, equal_nan=True)
 
 
+@pytest.mark.parametrize("name,step", [("symphony_rows", 5), ("pitchy_pl", 8), ("powerlaw", 8), ("pitchy_kappa", 10),
+                                       ("crank_pitchypl_64", 4)])
+def test_oracle_reproduces_the_fixtures_made_with_the_reference(oracle, golden, name, step):
+    """The fixtures were computed with the reference's own leung-bessel/src/bessel.c.  Whichever Bessel evaluator
+    this build links (oracle.bessel_source()), a strided sample of every fixture recomputed now must agree with them
+    to rounding, NaN pattern included: the standing check of oracle/leung_bessel.c against the reference."""
+    fx = golden(name)
+    rows = np.arange(0, len(fx["s"]), step)
+    out, lobes = oracle.batch(fx["kind"], fx["s"][rows], fx["theta"][rows], [np.asarray(p)[rows] for p in fx["params"]])
+    want = fx["out"][:, rows]
+    assert np.array_equal(np.isnan(out), np.isnan(want))
+    ok = ~np.isnan(want) & (want != 0)
+    rel = np.abs(out[ok] / want[ok] - 1)
+    assert np.median(rel) < 1e-14 and rel.max() < 1e-10, (np.median(rel), rel.max())
+    assert np.array_equal(out[~ok], want[~ok], equal_nan=True)
+
+
 # --- diagnostics of the Symphony double integral (src/lib.rs:249-299) ------------------------
 
 def test_symphony_diagnostics_are_mutually_consistent(oracle):
