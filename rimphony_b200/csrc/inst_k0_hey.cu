@@ -2,7 +2,8 @@
 #include "rb_kernels.cuh"
 namespace rbhost {
 template int stage_normalize<rb::kDistPowerLaw>(const BatchArgs &, int, cudaStream_t);
-template int stage_heyvaerts<rb::kDistPowerLaw>(const BatchArgs &, bool, int, cudaStream_t);
+template int stage_heyvaerts<rb::kDistPowerLaw, false>(const BatchArgs &, int, cudaStream_t);
+template int stage_heyvaerts<rb::kDistPowerLaw, true>(const BatchArgs &, int, cudaStream_t);
 template int stage_dist_eval<rb::kDistPowerLaw>(const double *, int, long long, const double *, const double *, double *,
                                        cudaStream_t);
 }

@@ -41,22 +41,15 @@
 #define RB_TABLE static const
 #endif
 
-#if defined(RB_HOST_EMU) && defined(RB_DEBUG_FAIL)
-#include <stdio.h>
-#define RB_TRACE_FAIL(what, c, lo, hi, x, y) \
-    fprintf(stderr, "qag fail: %s chan %d on [%.10g, %.10g] (%g, %g) NV=%d\n", what, c, lo, hi, x, y, NV)
-#else
-#define RB_TRACE_FAIL(what, c, lo, hi, x, y) ((void)0)
-#endif
-
 namespace rb {
 
 // Out-of-line double-precision transcendentals.  The product kernels are bound by instruction
 // fetch (profiles/): every inlined log/exp/cbrt costs 40-80 SASS instructions per call site, and
 // the hot loop has a dozen of them.  One shared copy each keeps the loop in the instruction cache.
 //
-// RB_LEAN_MATH (defined by the product-path translation units inst_k*_heyfast.cu / inst_k*_symfast.cu and by
-// the host harness; the QUADPACK-faithful kernels keep the CUDA library's functions): the kernels issue
+// RB_LEAN_MATH (defined by the Symphony translation units inst_k*_symfast.cu / inst_k*_sym.cu, by the product
+// Heyvaerts units inst_k*_heyfast.cu and by the host harness; only inst_k*_hey.cu, with the faithful Heyvaerts,
+// normalisation and dist_eval kernels, keep the CUDA library's functions): the kernels issue
 // 0.7-1.2 instructions per cycle and SM, every instruction counts the same, and ncu's source page says a
 // quarter of them is spent on IEEE-correct division (16 instructions each, 26-36 per node), on libdevice's
 // log/exp (87 / 64 instructions, two of every three of them moves of literal constants into uniform
@@ -152,9 +145,6 @@ inline double rb_rsqrt_seed(double x)
 #endif
 RB_FN double rb_sqrt(double x)
 {
-#ifdef RB_NO_LEAN_SQRT // tuning knob of the A/B in profiles/r02_instruction_work_ab.log (s15): the IEEE sequence
-    return sqrt(x);
-#endif
     const double y = rb_rsqrt_seed(x);
     double g = x * y, h = 0.5 * y;
     const double r = fma(-h, g, 0.5);
@@ -238,7 +228,7 @@ inline double rb_cbrt(double x) { return cbrt(x); }
 RB_FN double rb_rcp(double b) { return 1.0 / b; }
 RB_FN double rb_div(double a, double b) { return a / b; }
 RB_FN double rb_sqrt(double x) { return sqrt(x); }
-#if defined(RB_DEVICE_BUILD) && !defined(RB_INLINE_MATH) // measured: +9 % sets/s over inlining
+#ifdef RB_DEVICE_BUILD // measured: +9 % sets/s over inlining
 static __device__ __noinline__ double rb_log(double x) { return log(x); }
 static __device__ __noinline__ double rb_exp(double x) { return exp(x); }
 static __device__ __noinline__ double rb_cbrt(double x) { return cbrt(x); }
@@ -688,16 +678,12 @@ RB_FN void qag_joint(Warp &w, Apply &apply, int n_init, const double *bounds, do
             continue;
         const double tol = epsrel * fabs(area[c]);
         const double round_off = 50.0 * DBL_EPSILON * rabs0[c];
-        if (errsum[c] <= round_off && errsum[c] > tol) {
+        if (errsum[c] <= round_off && errsum[c] > tol)
             state[c] = kChanFailed; // GSL_EROUND on the first application
-            RB_TRACE_FAIL("first-application EROUND", c, bounds[0], bounds[n_init], errsum[c], tol);
-        }
         else if ((errsum[c] <= tol && errsum[c] != rasc0[c]) || errsum[c] == 0.0)
             state[c] = kChanDone;
-        else if (!(errsum[c] == errsum[c]) || !(area[c] == area[c])) {
+        else if (!(errsum[c] == errsum[c]) || !(area[c] == area[c]))
             state[c] = kChanFailed; // NaN integrand: GSL ends in EFAILED
-            RB_TRACE_FAIL("first-application NaN", c, bounds[0], bounds[n_init], errsum[c], area[c]);
-        }
         else
             n_active++;
     }
@@ -729,7 +715,6 @@ RB_FN void qag_joint(Warp &w, Apply &apply, int n_init, const double *bounds, do
         const int vw = Policy::val(cw);
         const int i_max = list_argmax<NV>(w, L, vw, Policy::side(cw), split);
         if (i_max < 0) {
-            RB_TRACE_FAIL("no interval", cw, bounds[0], bounds[n_init], errsum[cw], area[cw]);
             state[cw] = kChanFailed;
             n_active--;
             continue;
@@ -786,11 +771,9 @@ RB_FN void qag_joint(Warp &w, Apply &apply, int n_init, const double *bounds, do
                 state[c] = kChanDone;
                 n_active--;
             } else if (!(errsum[c] > tol)) {
-                RB_TRACE_FAIL("NaN in loop", c, a1, b2, errsum[c], area[c]);
                 state[c] = kChanFailed; // NaN
                 n_active--;
             } else if (c == cw && (rnd1[c] >= 6 || rnd2[c] >= 20 || too_small)) {
-                RB_TRACE_FAIL(too_small ? "ESING" : "EROUND", c, bounds[0], bounds[n_init], errsum[c], tol);
                 state[c] = kChanFailed; // GSL_EROUND / GSL_ESING
                 n_active--;
             }

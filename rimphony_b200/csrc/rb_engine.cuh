@@ -43,61 +43,6 @@ constexpr int kEngTile = 2 * kEngChan * kEngRow; // doubles per tile (A rows the
 constexpr unsigned kAppBudget = 150000; // rule applications per point after which every panel is accepted as is
                                         // (status CAP_HIT): bounds the cost of a point whose integral does not converge
 
-// --- lock-step pacing -------------------------------------------------------------------------
-// The product kernels are bound by instruction supply: a warp streams through ~40 KB of
-// straight-line code per rule application (6 KB L0 per scheduler, 32 KB L1.5 per SM), so with
-// every warp of a scheduler at its own place of that code each one pays for its own fetches.
-// With RB_LOCKSTEP the warps of a CTA (1) or of one scheduler (2: warps w, w + 4, w + 8, ...)
-// meet at a barrier before every rule application and before the seeding of every inner
-// integral, so that they run the same code at the same time and a fetched line serves all of
-// them.  The barrier carries no data; it only paces.  A warp that has run out of points keeps
-// arriving with idle = true until the whole group is idle (the popc the barrier returns).
-#ifndef RB_LOCKSTEP
-#define RB_LOCKSTEP 0
-#endif
-#if defined(RB_DEVICE_BUILD) && RB_LOCKSTEP
-// Mode 4: cohorts.  Warps that reach a tick at about the same time go on together, RB_LOCKSTEP_COHORT at a
-// time, whichever they are, and nobody waits for the slowest warp of the CTA (with modes 1 and 2 the
-// time lost at the barrier equals the instruction-fetch time it saves: profiles/r02_lockstep16_details.txt).
-// A hardware barrier cannot do this (its thread count must be met exactly; extra arrivals are undefined
-// behaviour and hang on sm_100a), so it is a ticket counter in shared memory: arrival t belongs to cohort
-// t / C, which is released once (arrivals + warps that have run out of points) reaches (t / C + 1) C.
-// A warp only ever waits for arrivals that are certain to come, so there is nothing to drain.
-#ifndef RB_LOCKSTEP_COHORT
-#define RB_LOCKSTEP_COHORT 8
-#endif
-#if RB_LOCKSTEP == 4
-static __shared__ int g_lockstep_state[2]; // [0] arrivals, [1] idle warps
-#endif
-RB_FN unsigned lockstep_group_threads()
-{
-    return (RB_LOCKSTEP == 2) ? blockDim.x >> 2 : blockDim.x;
-}
-RB_FN unsigned lockstep_tick(bool idle = false)
-{
-    unsigned r = 0;
-#if RB_LOCKSTEP == 4
-    if ((threadIdx.x & 31) == 0) {
-        volatile int *st = g_lockstep_state;
-        const int ticket = atomicAdd(&g_lockstep_state[0], 1);
-        const int target = (ticket / RB_LOCKSTEP_COHORT + 1) * RB_LOCKSTEP_COHORT;
-        while (st[0] + st[1] < target)
-            __nanosleep(40);
-    }
-    __syncwarp();
-    return r;
-#else
-    const unsigned id = (RB_LOCKSTEP == 2) ? 1u + ((threadIdx.x >> 5) & 3u) : 0u;
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %1, 0;\n\tbar.red.popc.u32 %0, %2, %3, p;\n\t}"
-                 : "=r"(r)
-                 : "r"((unsigned)idle), "r"(id), "r"(lockstep_group_threads()));
-    return r;
-#endif
-}
-#else
-RB_FN unsigned lockstep_tick(bool = false) { return 0; }
-#endif
-
 // per-warp shared-memory working set of one quadrature level; CH = channel rows of the tile (the Heyvaerts
 // kernel has two integrands: a quarter of the shared memory, which is what bounds its CTAs per SM)
 template <int CH>

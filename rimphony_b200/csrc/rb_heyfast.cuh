@@ -120,9 +120,6 @@ RB_FN_NOINLINE bool hey_inner_integral(Warp &w, const HeyFastCtx<KIND> &cx, int 
     const HeyGeometry &g = cx.g;
     PanelStack stk;
     stk.reset(&ws.inner);
-#ifndef RB_LOCKSTEP_NOSEED
-    lockstep_tick(); // a seeding tick
-#endif
 
     bool empty = false;
     // QR with pomega_max = sqrt(sigma^2 - sigma0^2): x -> 0 at both ends of the pomega range and the
@@ -239,7 +236,6 @@ RB_FN_NOINLINE bool hey_inner_integral(Warp &w, const HeyFastCtx<KIND> &cx, int 
         stk.pop(ta, tb, tag);
         const double tc = 0.5 * (ta + tb), thl = 0.5 * (tb - ta);
         warp_fence();
-        lockstep_tick(); // a rule-application tick
 #ifdef RB_DEVICE_BUILD
         {
             double vals[2];
@@ -307,9 +303,6 @@ RB_FN_NOINLINE bool hey_inner_integral(Warp &w, const HeyFastCtx<KIND> &cx, int 
             ok[c] = panel_ok(r[c], e[c], cx.epsrel_inner, kHeyInnerFloor * fmax(est[c] + fabs(r[c]), big[c]));
         }
         const bool accept = chan_all(ok, 2);
-#ifdef RB_TRACE_HEYINNER
-        RB_TRACE_HEYINNER(which, v, ta, tb, r, e, ok, sine_map);
-#endif
         if (accept || !stk.room(2) || panel_too_small(ta, tb) || w.n_apply_lanes > kAppBudget) {
             if (!accept && w.n_apply_lanes > kAppBudget)
                 w.status |= kStatusCapHit; // (a panel at the bisection floor is an integrable end-point singularity)
@@ -460,9 +453,6 @@ RB_FN_NOINLINE void hey_outer_integral(Warp &w, const HeyFastCtx<KIND> &cx, int 
             ok[c] = panel_ok(r[c], e[c], cx.epsrel_outer, fmax(fabs(scale[c]) + fabs(result[c]), big[c]));
         }
         bool accept = chan_all(ok, 2);
-#ifdef RB_TRACE_HEYFAST
-        RB_TRACE_HEYFAST(which, map, ta, tb, r, e, ok, w.n_apply_lanes);
-#endif
         // An outer panel that still fails kHeyOuterMaxDepth bisections below its seed sits next to
         // sigma = s, where the outer integrand behaves like |sigma - s|^(2 s - 1) (see kHeyRefDivergesV).
         // It is accepted as it is, with STATUS_CAP_HIT: the singularity is integrable and what is left
@@ -562,9 +552,6 @@ RB_FN_NOINLINE void hey_march(Warp &w, const HeyFastCtx<KIND> &cx, int which, do
         PerChan<double> contrib;
         hey_outer_integral<KIND>(w, cx, which, map, lo, hi, val, contrib, chan_all(minor, kEngChan));
         RB_FOR_CHAN(c, 2) { last[c] = contrib[c]; }
-#ifdef RB_TRACE_HEYMARCH
-        RB_TRACE_HEYMARCH(which, steps, lo, hi, delta, contrib, val);
-#endif
 
         RB_FOR_CHAN(c, 2)
         {

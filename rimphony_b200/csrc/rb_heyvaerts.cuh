@@ -58,7 +58,6 @@ struct HeyNode {
         // exactly 1 (or beyond) a few 1e-6 of the range before the end, and the pitch-angle factor
         // sin^k(xi), d f / d cos(xi) ~ 1 / sin^2(xi) turn into 0/0 there.
         double sin2 = NAN;
-#ifndef RB_NO_EXACT_SIN2
         if (x_exact == x_exact) {
             const double q = sigma - pomega * g.cos_th;
             const double xs = x * g.sin_th;
@@ -70,7 +69,6 @@ struct HeyNode {
             } else
                 sin2 = NAN;
         }
-#endif
 
         double f, dfdg, dfdcxi;
         dist_eval<KIND>(d, gamma, mu, f, dfdg, dfdcxi, sin2, sq);
@@ -285,13 +283,7 @@ RB_FN_NOINLINE void hey_step_outward(Warp &w, Outer &F, IntervalList<NV> &olist,
 
         const double bounds[2] = {dir > 0 ? edge : edge - delta, dir > 0 ? edge + delta : edge};
         double contrib[NV];
-#ifdef RB_TRACE_HEY
-        const unsigned apps0_ = w.n_apply_lanes;
-#endif
         qag_joint<PolicyPlain<NV>>(w, ap, 1, bounds, epsrel_outer, olist, keep, contrib);
-#ifdef RB_TRACE_HEY
-        RB_TRACE_HEY("step", bounds[0], bounds[1], contrib, val, w.n_apply_lanes - apps0_, olist.size);
-#endif
 
 #pragma unroll
         for (int c = 0; c < NV; c++) {
@@ -345,9 +337,6 @@ RB_FN void heyvaerts_point(Warp &w, const Dist &dist, double s, double theta, do
             ApplySeq<NV, HeyNROuter<KIND, NV>> ap{nr};
             const double bounds[2] = {-3.0 * geom.sigma0, 3.0 * geom.sigma0};
             qag_joint<PolicyPlain<NV>>(w, ap, 1, bounds, epsrel_outer, olist, all, nr_val);
-#ifdef RB_TRACE_HEY
-            RB_TRACE_HEY("init", bounds[0], bounds[1], nr_val, nr_val, w.n_apply_lanes, olist.size);
-#endif
 #pragma unroll
             for (int c = 0; c < NV; c++)
                 if (!(nr_val[c] == nr_val[c]))

@@ -36,6 +36,40 @@ __global__ void __launch_bounds__(kThreadsPerBlock) k_normalize(BatchArgs a)
     }
 }
 
+// Lane 0's write-back of one point: the requested coefficient slots FIRST.. of out8, the lobes
+// (Symphony only: `lobes4` is null for Heyvaerts), the work-counter row of the kernel and the
+// status bits, in that order (writing the lobes first changes the register allocation of k_symphony_fast).
+// CONTINUATION: the kernel may run as the faithful continuation of the product kernel
+// (a.from_reroute_list), whose rule applications go on top of what the product kernel counted.
+template <int FIRST, bool CONTINUATION = false, int NC>
+__device__ __forceinline__ void write_point(const BatchArgs &a, const Warp &w, long long i, const double (&out)[NC],
+                                            const double *lobes4)
+{
+    bool any_nan = false;
+#pragma unroll
+    for (int c = 0; c < NC; c++) {
+        if ((a.coeff_mask >> (FIRST + c)) & 1u) {
+            a.out8[(long long)(FIRST + c) * a.n + i] = out[c];
+            any_nan |= !(out[c] == out[c]);
+        }
+    }
+    if (lobes4 && a.lobes4) {
+#pragma unroll
+        for (int c = 0; c < 4; c++)
+            a.lobes4[(long long)c * a.n + i] = lobes4[c];
+    }
+    if (a.counters) {
+        unsigned *row = a.counters + (FIRST ? a.n : 0);
+        if (CONTINUATION && a.from_reroute_list)
+            atomicAdd(&row[i], w.n_apply_lanes);
+        else
+            row[i] = w.n_apply_lanes;
+    }
+    const unsigned st = w.status | (any_nan ? kStatusNaN : 0u);
+    if (a.status && st)
+        atomicOr(&a.status[i], (int)st);
+}
+
 template <int KIND, bool FUSED>
 __global__ void __launch_bounds__(kThreadsPerBlock, FUSED ? 3 : 4) k_symphony(BatchArgs a)
 {
@@ -118,30 +152,8 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FUSED ? 3 : 4) k_symphony(Ba
             symphony_point<KIND, FUSED, kSymGammaCap, kSymNCap>(w, d, a.s[i], a.theta[i], a.eps_gamma, a.eps_n, ws,
                                                                 out6, lobes4);
 
-        if (w.lane == 0) {
-            bool any_nan = false;
-#pragma unroll
-            for (int c = 0; c < 6; c++) {
-                if ((a.coeff_mask >> c) & 1u) {
-                    a.out8[(long long)c * a.n + i] = out6[c];
-                    any_nan |= !(out6[c] == out6[c]);
-                }
-            }
-            if (a.lobes4) {
-#pragma unroll
-                for (int c = 0; c < 4; c++)
-                    a.lobes4[(long long)c * a.n + i] = lobes4[c];
-            }
-            if (a.counters) {
-                if (a.from_reroute_list)
-                    atomicAdd(&a.counters[i], w.n_apply_lanes); // on top of what the product kernel counted
-                else
-                    a.counters[i] = w.n_apply_lanes;
-            }
-            const unsigned st = w.status | (any_nan ? kStatusNaN : 0u);
-            if (a.status && st)
-                atomicOr(&a.status[i], (int)st);
-        }
+        if (w.lane == 0)
+            write_point<0, true>(a, w, i, out6, lobes4);
     }
 }
 
@@ -177,49 +189,16 @@ __global__ void __launch_bounds__(kThreadsPerBlock, 4) k_symphony_diag(BatchArgs
     }
 }
 
-#ifndef RB_FAST_BLOCKS
-#define RB_FAST_BLOCKS 5 // resident CTAs per SM the product kernels are compiled for (96 registers; +5 % over 4)
-#endif
-#ifndef RB_HEY_BLOCKS
-#define RB_HEY_BLOCKS 8 // the Heyvaerts kernel (64 registers; its tiles have two channel rows, 14 KB per CTA).  5 -> 8 CTAs per SM: -13 % kernel time; 10 (48 registers) is as fast but its 768 B of stack per thread x 1280 threads x 148 SMs no longer fit the L2 and 0.7 MB per point go to DRAM (0.1 MB at 8)
-#endif
-#ifndef RB_FAST_WARPS
-#define RB_FAST_WARPS 4 // warps per CTA of the product kernels
-#endif
-constexpr int kFastWarps = RB_FAST_WARPS;
+constexpr int kFastBlocks = 5; // resident CTAs per SM the product kernels are compiled for (96 registers; +5 % over 4)
+constexpr int kHeyBlocks = 8;  // the Heyvaerts kernel (64 registers; its tiles have two channel rows, 14 KB per CTA).  5 -> 8 CTAs per SM: -13 % kernel time; 10 (48 registers) is as fast but its 768 B of stack per thread x 1280 threads x 148 SMs no longer fit the L2 and 0.7 MB per point go to DRAM (0.1 MB at 8)
+constexpr int kFastWarps = 4;  // warps per CTA of the product kernels
 constexpr int kFastThreads = kFastWarps * 32;
-static_assert(RB_LOCKSTEP != 2 || kFastWarps % 4 == 0, "per-scheduler lock-step groups need a multiple of four warps");
-// Lock-step bookkeeping of a CTA (cohort mode keeps two counters in shared memory).
-__device__ __forceinline__ void lockstep_init()
-{
-#if RB_LOCKSTEP == 4
-    if (threadIdx.x == 0) {
-        g_lockstep_state[0] = 0;
-        g_lockstep_state[1] = 0;
-    }
-    __syncthreads();
-#endif
-}
-
-// After its last point: barrier modes keep the barrier company until the whole group is idle; cohort
-// mode just counts the warp out.
-__device__ __forceinline__ void lockstep_drain()
-{
-#if RB_LOCKSTEP == 4
-    if ((threadIdx.x & 31) == 0)
-        atomicAdd(&g_lockstep_state[1], 1);
-#elif RB_LOCKSTEP
-    while (lockstep_tick(true) != lockstep_group_threads()) {
-    }
-#endif
-}
 
 // The product path: compact engine (rb_engine.cuh, rb_symfast.cuh).
 template <int KIND>
-__global__ void __launch_bounds__(kFastThreads, RB_FAST_BLOCKS) k_symphony_fast(BatchArgs a)
+__global__ void __launch_bounds__(kFastThreads, kFastBlocks) k_symphony_fast(BatchArgs a)
 {
     extern __shared__ double smem[];
-    lockstep_init();
     const int warp = threadIdx.x >> 5;
     SymFastWS &ws = reinterpret_cast<SymFastWS *>(smem)[warp];
     Warp w;
@@ -259,28 +238,9 @@ __global__ void __launch_bounds__(kFastThreads, RB_FAST_BLOCKS) k_symphony_fast(
             continue;
         }
 
-        if (w.lane == 0) {
-            bool any_nan = false;
-#pragma unroll
-            for (int c = 0; c < 6; c++) {
-                if ((a.coeff_mask >> c) & 1u) {
-                    a.out8[(long long)c * a.n + i] = out6[c];
-                    any_nan |= !(out6[c] == out6[c]);
-                }
-            }
-            if (a.lobes4) {
-#pragma unroll
-                for (int c = 0; c < 4; c++)
-                    a.lobes4[(long long)c * a.n + i] = lobes4[c];
-            }
-            if (a.counters)
-                a.counters[i] = w.n_apply_lanes;
-            const unsigned st = w.status | (any_nan ? kStatusNaN : 0u);
-            if (a.status && st)
-                atomicOr(&a.status[i], (int)st);
-        }
+        if (w.lane == 0)
+            write_point<0>(a, w, i, out6, lobes4);
     }
-    lockstep_drain();
 }
 
 template <int KIND, bool FUSED>
@@ -313,30 +273,16 @@ __global__ void __launch_bounds__(kThreadsPerBlock, 4) k_heyvaerts(BatchArgs a)
         heyvaerts_point<KIND, FUSED, kHeyInnerCap, kHeyOuterCap>(w, d, s, theta, a.eps_hey_inner, a.eps_hey_outer, ws,
                                                                  out2);
 
-        if (w.lane == 0) {
-            bool any_nan = false;
-#pragma unroll
-            for (int c = 0; c < 2; c++) {
-                if ((a.coeff_mask >> (6 + c)) & 1u) {
-                    a.out8[(long long)(6 + c) * a.n + i] = out2[c];
-                    any_nan |= !(out2[c] == out2[c]);
-                }
-            }
-            if (a.counters)
-                a.counters[a.n + i] = w.n_apply_lanes;
-            const unsigned st = w.status | (any_nan ? kStatusNaN : 0u);
-            if (a.status && st)
-                atomicOr(&a.status[i], (int)st);
-        }
+        if (w.lane == 0)
+            write_point<6>(a, w, i, out2, nullptr);
     }
 }
 
 // The product path for rho_Q, rho_V: compact engine (rb_engine.cuh, rb_heyfast.cuh).
 template <int KIND>
-__global__ void __launch_bounds__(kFastThreads, RB_HEY_BLOCKS) k_heyvaerts_fast(BatchArgs a)
+__global__ void __launch_bounds__(kFastThreads, kHeyBlocks) k_heyvaerts_fast(BatchArgs a)
 {
     extern __shared__ double smem[];
-    lockstep_init();
     const int warp = threadIdx.x >> 5;
     HeyFastWS &ws = reinterpret_cast<HeyFastWS *>(smem)[warp];
     Warp w;
@@ -358,23 +304,9 @@ __global__ void __launch_bounds__(kFastThreads, RB_HEY_BLOCKS) k_heyvaerts_fast(
         double out2[2];
         heyvaerts_point_fast<KIND>(w, d, a.s[i], a.theta[i], a.eps_hey_inner, a.eps_hey_outer, ws, out2);
 
-        if (w.lane == 0) {
-            bool any_nan = false;
-#pragma unroll
-            for (int c = 0; c < 2; c++) {
-                if ((a.coeff_mask >> (6 + c)) & 1u) {
-                    a.out8[(long long)(6 + c) * a.n + i] = out2[c];
-                    any_nan |= !(out2[c] == out2[c]);
-                }
-            }
-            if (a.counters)
-                a.counters[a.n + i] = w.n_apply_lanes;
-            const unsigned st = w.status | (any_nan ? kStatusNaN : 0u);
-            if (a.status && st)
-                atomicOr(&a.status[i], (int)st);
-        }
+        if (w.lane == 0)
+            write_point<6>(a, w, i, out2, nullptr);
     }
-    lockstep_drain();
 }
 
 template <int KIND>
@@ -394,102 +326,66 @@ __global__ void k_dist_eval(Dist d, long long count, const double *gamma, const 
 // ---------------------------------------------------------------------------
 // stage launchers
 
-template <int KIND>
-int stage_normalize(const BatchArgs &a, int sm_count, cudaStream_t st)
+// One persistent launch: every CTA slot the device holds at once (`threads` per CTA, `smem` bytes of
+// dynamic shared memory each), but no more CTAs than `max_ctas` when that is positive.
+template <class... P, class... A>
+int launch_persistent(void (*kernel)(P...), size_t smem, int threads, long long max_ctas, int sm_count, cudaStream_t st,
+                      const A &...args)
 {
-    const size_t smem = (size_t)kWarpsPerBlock * kNormCap * IntervalList<1>::doubles_per_interval * sizeof(double);
-    int grid = 0;
-    if (set_smem(k_normalize<KIND>, smem) || persistent_grid(k_normalize<KIND>, smem, sm_count, &grid))
-        return 1;
-    const long long need = (a.n + kWarpsPerBlock - 1) / kWarpsPerBlock;
-    if (need < grid)
-        grid = (int)need;
-    k_normalize<KIND><<<grid, kThreadsPerBlock, smem, st>>>(a);
+    RB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    RB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+    if (per_sm < 1)
+        return fail("kernel does not fit on an SM (smem %zu)", smem);
+    int grid = per_sm * sm_count; // a multiple of the SM count
+    if (max_ctas > 0 && max_ctas < grid)
+        grid = (int)max_ctas;
+    kernel<<<grid, threads, smem, st>>>(args...);
     g_launches++;
     RB_CUDA(cudaGetLastError());
     return 0;
 }
 
 template <int KIND>
-int stage_symphony(const BatchArgs &a, bool faithful, int sm_count, cudaStream_t st)
+int stage_normalize(const BatchArgs &a, int sm_count, cudaStream_t st)
 {
-    int grid = 0;
-    if (faithful) {
-        const size_t smem = kWarpsPerBlock * sizeof(SymWorkspace<false, kSymGammaCap, kSymNCap>);
-        if (set_smem(k_symphony<KIND, false>, smem) || persistent_grid(k_symphony<KIND, false>, smem, sm_count, &grid))
-            return 1;
-        k_symphony<KIND, false><<<grid, kThreadsPerBlock, smem, st>>>(a);
-    } else {
-        const size_t smem = kWarpsPerBlock * sizeof(SymWorkspace<true, kSymGammaCap, kSymNCap>);
-        if (set_smem(k_symphony<KIND, true>, smem) || persistent_grid(k_symphony<KIND, true>, smem, sm_count, &grid))
-            return 1;
-        k_symphony<KIND, true><<<grid, kThreadsPerBlock, smem, st>>>(a);
-    }
-    g_launches++;
-    RB_CUDA(cudaGetLastError());
-    return 0;
+    const size_t smem = (size_t)kWarpsPerBlock * kNormCap * IntervalList<1>::doubles_per_interval * sizeof(double);
+    return launch_persistent(k_normalize<KIND>, smem, kThreadsPerBlock, (a.n + kWarpsPerBlock - 1) / kWarpsPerBlock,
+                             sm_count, st, a);
+}
+
+template <int KIND, bool FUSED>
+int stage_symphony(const BatchArgs &a, int sm_count, cudaStream_t st)
+{
+    const size_t smem = kWarpsPerBlock * sizeof(SymWorkspace<FUSED, kSymGammaCap, kSymNCap>);
+    return launch_persistent(k_symphony<KIND, FUSED>, smem, kThreadsPerBlock, 0, sm_count, st, a);
 }
 
 template <int KIND>
 int stage_symphony_diag(const BatchArgs &a, const DiagArgs &g, int sm_count, cudaStream_t st)
 {
-    int grid = 0;
     const size_t smem = kWarpsPerBlock * sizeof(SymWorkspace<false, kSymGammaCap, kSymNCap>);
-    if (set_smem(k_symphony_diag<KIND>, smem) || persistent_grid(k_symphony_diag<KIND>, smem, sm_count, &grid))
-        return 1;
-    const long long need = (g.count + kWarpsPerBlock - 1) / kWarpsPerBlock;
-    if (need < grid)
-        grid = (int)need;
-    k_symphony_diag<KIND><<<grid, kThreadsPerBlock, smem, st>>>(a, g);
-    g_launches++;
-    RB_CUDA(cudaGetLastError());
-    return 0;
+    return launch_persistent(k_symphony_diag<KIND>, smem, kThreadsPerBlock, (g.count + kWarpsPerBlock - 1) / kWarpsPerBlock,
+                             sm_count, st, a, g);
 }
 
 template <int KIND>
 int stage_symphony_fast(const BatchArgs &a, int sm_count, cudaStream_t st)
 {
-    int grid = 0;
-    const size_t smem = kFastWarps * sizeof(SymFastWS);
-    if (set_smem(k_symphony_fast<KIND>, smem) || persistent_grid(k_symphony_fast<KIND>, smem, sm_count, &grid, kFastThreads))
-        return 1;
-    k_symphony_fast<KIND><<<grid, kFastThreads, smem, st>>>(a);
-    g_launches++;
-    RB_CUDA(cudaGetLastError());
-    return 0;
+    return launch_persistent(k_symphony_fast<KIND>, kFastWarps * sizeof(SymFastWS), kFastThreads, 0, sm_count, st, a);
 }
 
-template <int KIND>
-int stage_heyvaerts(const BatchArgs &a, bool fused, int sm_count, cudaStream_t st)
+template <int KIND, bool FUSED>
+int stage_heyvaerts(const BatchArgs &a, int sm_count, cudaStream_t st)
 {
-    int grid = 0;
-    if (!fused) {
-        const size_t smem = kWarpsPerBlock * sizeof(HeyWorkspace<false, kHeyInnerCap, kHeyOuterCap>);
-        if (set_smem(k_heyvaerts<KIND, false>, smem) || persistent_grid(k_heyvaerts<KIND, false>, smem, sm_count, &grid))
-            return 1;
-        k_heyvaerts<KIND, false><<<grid, kThreadsPerBlock, smem, st>>>(a);
-    } else {
-        const size_t smem = kWarpsPerBlock * sizeof(HeyWorkspace<true, kHeyInnerCap, kHeyOuterCap>);
-        if (set_smem(k_heyvaerts<KIND, true>, smem) || persistent_grid(k_heyvaerts<KIND, true>, smem, sm_count, &grid))
-            return 1;
-        k_heyvaerts<KIND, true><<<grid, kThreadsPerBlock, smem, st>>>(a);
-    }
-    g_launches++;
-    RB_CUDA(cudaGetLastError());
-    return 0;
+    const size_t smem = kWarpsPerBlock * sizeof(HeyWorkspace<FUSED, kHeyInnerCap, kHeyOuterCap>);
+    return launch_persistent(k_heyvaerts<KIND, FUSED>, smem, kThreadsPerBlock, 0, sm_count, st, a);
 }
 
 template <int KIND>
 int stage_heyvaerts_fast(const BatchArgs &a, int sm_count, cudaStream_t st)
 {
-    int grid = 0;
-    const size_t smem = kFastWarps * sizeof(HeyFastWS);
-    if (set_smem(k_heyvaerts_fast<KIND>, smem) || persistent_grid(k_heyvaerts_fast<KIND>, smem, sm_count, &grid, kFastThreads))
-        return 1;
-    k_heyvaerts_fast<KIND><<<grid, kFastThreads, smem, st>>>(a);
-    g_launches++;
-    RB_CUDA(cudaGetLastError());
-    return 0;
+    return launch_persistent(k_heyvaerts_fast<KIND>, kFastWarps * sizeof(HeyFastWS), kFastThreads, 0, sm_count, st, a);
 }
 
 template <int KIND>

@@ -1,6 +1,7 @@
-// rb_launch.cuh -- kernels and per-stage launchers shared by the translation
-// units of the product library (the kernels are instantiated per distribution
-// kind in inst_*.cu so that they compile in parallel).
+// rb_launch.cuh -- launch geometry, kernel arguments and the per-stage launcher
+// declarations shared by the translation units of the product library.  The
+// kernels and launchers are in rb_kernels.cuh, instantiated per distribution kind
+// in inst_*.cu so that they compile in parallel.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -127,36 +128,18 @@ extern std::atomic<uint64_t> g_launches;
             return ::rbhost::fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
     } while (0)
 
-template <class K>
-int set_smem(K kernel, size_t bytes)
-{
-    RB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    return 0;
-}
-
-template <class K>
-int persistent_grid(K kernel, size_t smem, int sm_count, int *grid, int threads = kThreadsPerBlock)
-{
-    int per_sm = 0;
-    RB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
-    if (per_sm < 1)
-        return ::rbhost::fail("kernel does not fit on an SM (smem %zu)", smem);
-    *grid = per_sm * sm_count; // every resident CTA slot, a multiple of the SM count
-    return 0;
-}
-
 // Per-stage launchers, explicitly instantiated in inst_*.cu.
 template <int KIND>
 int stage_normalize(const BatchArgs &a, int sm_count, cudaStream_t st);
-template <int KIND>
-int stage_symphony(const BatchArgs &a, bool faithful, int sm_count, cudaStream_t st);
+template <int KIND, bool FUSED>
+int stage_symphony(const BatchArgs &a, int sm_count, cudaStream_t st);
 int stage_classify(const BatchArgs &a, cudaStream_t st);
 template <int KIND>
 int stage_symphony_fast(const BatchArgs &a, int sm_count, cudaStream_t st);
 template <int KIND>
 int stage_symphony_diag(const BatchArgs &a, const DiagArgs &g, int sm_count, cudaStream_t st);
-template <int KIND>
-int stage_heyvaerts(const BatchArgs &a, bool fused, int sm_count, cudaStream_t st);
+template <int KIND, bool FUSED>
+int stage_heyvaerts(const BatchArgs &a, int sm_count, cudaStream_t st);
 template <int KIND>
 int stage_heyvaerts_fast(const BatchArgs &a, int sm_count, cudaStream_t st);
 template <int KIND>

@@ -49,10 +49,7 @@ constexpr int kMaxChunks = 400;   // safety net of the chunk loop (the reference
 // points (hard kappa spectra) are not computed here: they are flagged and re-run with the
 // reference's exact sequence of rule applications (MODE_FAITHFUL kernel).
 constexpr double kSensitiveN = 5e9;
-#ifndef RB_SENSITIVE_FRACTION
-#define RB_SENSITIVE_FRACTION 5e-4 // per chunk; the chunks above decay at least like 1/2 per decade: < 1e-3 in all
-#endif
-constexpr double kSensitiveFraction = RB_SENSITIVE_FRACTION;
+constexpr double kSensitiveFraction = 5e-4; // per chunk; the chunks above decay at least like 1/2 per decade: < 1e-3 in all
 // A flagged point does not start over: up to n ~ 1e9 the reference's quadrature is sound and
 // the product path reproduces it, so the faithful sequence resumes from the chunk-loop state
 // recorded at the first chunk starting beyond kHandoverN (s >= 10, where the chunk sequence
@@ -247,9 +244,6 @@ RB_FN_NOINLINE void sym_gamma_integral(Warp &w, const SymFastCtx<KIND> &cx, doub
         }
     }
 
-#ifndef RB_LOCKSTEP_NOSEED
-    lockstep_tick(); // a seeding tick
-#endif
     warp_fence();
 #ifdef RB_DEVICE_BUILD
     if (w.lane < 2) // orders n and n + 1 side by side
@@ -461,7 +455,6 @@ RB_FN_NOINLINE void sym_gamma_integral(Warp &w, const SymFastCtx<KIND> &cx, doub
             tb0 = mid;
         }
         warp_fence(); // the previous reduce has finished reading the tile
-        lockstep_tick(); // a rule-application tick
 
 #ifdef RB_DEVICE_BUILD
         {
@@ -502,9 +495,6 @@ RB_FN_NOINLINE void sym_gamma_integral(Warp &w, const SymFastCtx<KIND> &cx, doub
                                  kInnerFloor * fmax(est[c] + fabs(r[c]), big[c]));
             }
             const bool accept = chan_all(ok, 6);
-#ifdef RB_TRACE_INNER
-            RB_TRACE_INNER(n, ta, tb, r, e, ok, est);
-#endif
             if (accept || !stk.room(2) || panel_too_small(ta, tb) || w.n_apply_lanes > kAppBudget) {
                 if (!accept && w.n_apply_lanes > kAppBudget)
                     w.status |= kStatusCapHit; // (a panel at the bisection floor is an integrable end-point singularity)
@@ -525,9 +515,6 @@ RB_FN_NOINLINE void sym_gamma_integral(Warp &w, const SymFastCtx<KIND> &cx, doub
         stk.seal();
     }
 
-#ifdef RB_TRACE_GEND
-    RB_TRACE_GEND(n, w.n_apply_lanes);
-#endif
     // add the eight accumulators to the sums of the outer rule
     (void)col;
     warp_fence();
@@ -871,9 +858,6 @@ RB_FN void symphony_point_fast(Warp &w, const Dist &dist, double s, double theta
                 ok[c] = !active[c] || panel_ok(r[c], e[c], epsrel_n, fabs(disc[c] + tail[c] + chunk[c]));
             }
             const bool accept = chan_all(ok, kEngChan);
-#ifdef RB_TRACE_FAST
-            RB_TRACE_FAST(chunk_no, ua, ub, r, e, ok, tail, chunk, w.n_apply_lanes);
-#endif
             if (accept || !stk.room(2) || panel_too_small(ua, ub) || w.n_apply_lanes > kAppBudget) {
                 if (!accept)
                     w.status |= kStatusCapHit;
@@ -885,9 +869,6 @@ RB_FN void symphony_point_fast(Warp &w, const Dist &dist, double s, double theta
             }
         }
 
-#ifdef RB_TRACE_CHUNK
-        RB_TRACE_CHUNK(chunk_no, light, n_lo_chunk, delta_n, chunk, tail, disc, w.n_apply_lanes);
-#endif
         if (n_lo_chunk >= kSensitiveN && s < 1e6) {
             // Fidelity guard, per accumulator: one whose chunks up here still matter leaves this
             // path (it is the emission coefficients of hard spectra, as a rule; absorption and

@@ -136,21 +136,12 @@ struct SymGammaIntegral {
         }
         warp_fence();
 
-#ifdef RB_TRACE_G
-        const unsigned apps_before = w.n_apply_lanes;
-#endif
-#ifdef RB_TRACE_GF
-        const unsigned apps_before_f = w.n_apply_lanes;
-#endif
         SymGammaIntegrand<KIND, NV> f{d, g, ord, n, 0};
         ApplyLanes<NV, SymGammaIntegrand<KIND, NV>> ap{f};
 
         if constexpr (FUSED) {
             const double bounds[3] = {gamma_minus_high, gamma_peak, gamma_plus_high};
             qag_joint<PolicySymphonySplit>(w, ap, 2, bounds, epsrel, *list, want, out);
-#ifdef RB_TRACE_G
-            RB_TRACE_G(n, w.n_apply_lanes - apps_before, out);
-#endif
         } else {
             f.sel = PolicySymphonySplit::val(sel);
             double bounds[2];
@@ -165,9 +156,6 @@ struct SymGammaIntegral {
                 bounds[1] = gamma_peak;
             }
             qag_joint<PolicyPlain<1>>(w, ap, 1, bounds, epsrel, *list, 1u, out);
-#ifdef RB_TRACE_GF
-            RB_TRACE_GF(n, sel, w.n_apply_lanes - apps_before_f, out[0]);
-#endif
         }
     }
 };

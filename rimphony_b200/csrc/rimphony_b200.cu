@@ -1,12 +1,15 @@
-// rimphony_b200.cu -- sm_100a kernels and the C ABI (include/rimphony_b200.h).
+// rimphony_b200.cu -- the C ABI (include/rimphony_b200.h) and its host side.
 //
-// Three persistent, warp-per-point kernels per distribution kind:
-//   k_normalize   full_calculation(): the normalisation constant of each point
-//   k_symphony    j_I, alpha_I, j_Q, alpha_Q, j_V, alpha_V       (rb_symphony.cuh)
-//   k_heyvaerts   rho_Q, rho_V                                    (rb_heyvaerts.cuh)
-// Points are independent, their cost varies by more than 10x, so each warp
-// pulls the next point from a global atomic counter.  All arithmetic is FP64 on
-// the CUDA cores; there is no dense contraction for the tensor cores to do.
+// A batch runs these kernels (rb_kernels.cuh, instantiated per distribution kind in inst_*.cu):
+//   k_normalize        full_calculation(): the normalisation constant of each point
+//   k_classify         the cost-ordered schedule of the two product kernels (this file)
+//   k_symphony_fast    j_I, alpha_I, j_Q, alpha_Q, j_V, alpha_V       (rb_symfast.cuh)
+//   k_heyvaerts_fast   rho_Q, rho_V                                    (rb_heyfast.cuh)
+// That is MODE_FAST, the default.  k_symphony (rb_symphony.cuh) computes the points k_symphony_fast
+// hands over to the reference's exact rule sequence; it and k_heyvaerts (rb_heyvaerts.cuh) replace
+// the product kernels in the other modes.  Points are independent, their cost varies by more than
+// 10x, so each warp of the persistent kernels pulls the next point from a global atomic counter.
+// All arithmetic is FP64 on the CUDA cores; there is no dense contraction for the tensor cores to do.
 //
 // There is deliberately no host implementation behind these entry points: with
 // no usable CUDA device every call fails with a nonzero return code.
@@ -19,6 +22,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/rimphony_b200.h"
@@ -254,17 +258,32 @@ int check_params(int kind, int n_params)
     return fail("unknown distribution kind %d", kind);
 }
 
+// The argument checks of the batched entry points; nonzero means a bad argument (the message is
+// set).  With n == 0 there is nothing to compute and nothing more to check; otherwise *o is resolved.
+int check_batch(int kind, int64_t n, const double *s, const double *theta, const double *const *params, int n_params,
+                const double *out8, const rimphony_b200_options *opts, ResolvedOptions *o)
+{
+    if (n < 0)
+        return fail("n_points is negative");
+    if (check_params(kind, n_params))
+        return 1;
+    if (n == 0)
+        return 0;
+    if (!s || !theta || !params || !out8)
+        return fail("null array pointer");
+    *o = resolve(opts);
+    if (o->mode < 0 || o->mode > 3)
+        return fail("unknown mode %d", o->mode);
+    return 0;
+}
+
 template <int KIND>
 int launch_kind(DeviceContext &c, BatchArgs a, const ResolvedOptions &o, cudaStream_t user_stream)
 {
     cudaStream_t st = user_stream ? user_stream : c.stream;
     // Heyvaerts always runs on the library's second stream, forked from and joined back
     // into `st` with events, so a caller-supplied stream keeps its ordering semantics.
-    cudaStream_t st_hey = c.stream_hey;
-    // tuning knob (tools/variant_bench.py): both stages on one stream, one after the other
-    static const bool serial_stages = getenv("RIMPHONY_B200_SERIAL_STAGES") != nullptr;
-    if (serial_stages)
-        st_hey = st;
+    const cudaStream_t st_hey = c.stream_hey;
     unsigned long long *counters = static_cast<unsigned long long *>(c.counters.ptr);
     const bool faithful = (o.mode == RIMPHONY_B200_MODE_FAITHFUL);
     const bool want_sym = (o.coeff_mask & 0x3Fu) != 0;
@@ -280,8 +299,7 @@ int launch_kind(DeviceContext &c, BatchArgs a, const ResolvedOptions &o, cudaStr
     if (o.mode == RIMPHONY_B200_MODE_FAST && stage_classify(a, st))
         return 1;
     RB_CUDA(cudaEventRecord(c.ev[1], st));
-    if (st_hey != st)
-        RB_CUDA(cudaStreamWaitEvent(st_hey, c.ev[1], 0));
+    RB_CUDA(cudaStreamWaitEvent(st_hey, c.ev[1], 0));
 
     // 2. Symphony
     if (want_sym) {
@@ -295,9 +313,10 @@ int launch_kind(DeviceContext &c, BatchArgs a, const ResolvedOptions &o, cudaStr
             b.next = counters + 0; // reused: reset between the two kernels
             RB_CUDA(cudaMemsetAsync(counters + 0, 0, sizeof(unsigned long long), st));
             b.from_reroute_list = 1;
-            if (stage_symphony<KIND>(b, true, c.sm_count, st))
+            if (stage_symphony<KIND, false>(b, c.sm_count, st))
                 return 1;
-        } else if (stage_symphony<KIND>(a, faithful, c.sm_count, st))
+        } else if (faithful ? stage_symphony<KIND, false>(a, c.sm_count, st)
+                            : stage_symphony<KIND, true>(a, c.sm_count, st))
             return 1;
     }
     RB_CUDA(cudaEventRecord(c.ev[2], st));
@@ -317,7 +336,7 @@ int launch_kind(DeviceContext &c, BatchArgs a, const ResolvedOptions &o, cudaStr
             b.next = counters + 1;
             b.sigma0_lo = -INFINITY;
             b.sigma0_hi = split;
-            if (stage_heyvaerts<KIND>(b, false, c.sm_count, st_hey))
+            if (stage_heyvaerts<KIND, false>(b, c.sm_count, st_hey))
                 return 1;
         }
         if (split < INFINITY) { // h and f on shared nodes for sigma0 >= split
@@ -325,38 +344,31 @@ int launch_kind(DeviceContext &c, BatchArgs a, const ResolvedOptions &o, cudaStr
             b.next = counters + 2;
             b.sigma0_lo = split;
             b.sigma0_hi = INFINITY;
-            if (stage_heyvaerts<KIND>(b, true, c.sm_count, st_hey))
+            if (stage_heyvaerts<KIND, true>(b, c.sm_count, st_hey))
                 return 1;
         }
     }
     RB_CUDA(cudaEventRecord(c.ev[4], st_hey));
-    if (st_hey != st)
-        RB_CUDA(cudaStreamWaitEvent(st, c.ev[4], 0));
+    RB_CUDA(cudaStreamWaitEvent(st, c.ev[4], 0));
     RB_CUDA(cudaEventRecord(c.ev[5], st));
     return 0;
 }
 
-int launch(DeviceContext &c, int kind, const BatchArgs &a, const ResolvedOptions &o, cudaStream_t user_stream)
+// Runs f(std::integral_constant<int, KIND>) for the distribution kind of the C ABI.
+template <class F>
+int dispatch_kind(int kind, F &&f)
 {
     switch (kind) {
     case RIMPHONY_B200_POWER_LAW:
-        return launch_kind<kDistPowerLaw>(c, a, o, user_stream);
+        return f(std::integral_constant<int, kDistPowerLaw>{});
     case RIMPHONY_B200_THERMAL_JUETTNER:
-        return launch_kind<kDistThermalJuettner>(c, a, o, user_stream);
+        return f(std::integral_constant<int, kDistThermalJuettner>{});
     case RIMPHONY_B200_PITCHY_PL:
-        return launch_kind<kDistPitchyPL>(c, a, o, user_stream);
+        return f(std::integral_constant<int, kDistPitchyPL>{});
     case RIMPHONY_B200_PITCHY_KAPPA:
-        return launch_kind<kDistPitchyKappa>(c, a, o, user_stream);
+        return f(std::integral_constant<int, kDistPitchyKappa>{});
     }
     return fail("unknown distribution kind %d", kind);
-}
-
-template <int KIND>
-int diag_kind(DeviceContext &c, const BatchArgs &a, const DiagArgs &g)
-{
-    if (stage_normalize<KIND>(a, c.sm_count, c.stream))
-        return 1;
-    return stage_symphony_diag<KIND>(a, g, c.sm_count, c.stream);
 }
 
 int collect_times(DeviceContext &c)
@@ -432,7 +444,7 @@ int run_device(int kind, int64_t n, const double *s, const double *theta, const 
         RB_CUDA(cudaStreamWaitEvent(st, c.ev_done, 0));
     if (status)
         RB_CUDA(cudaMemsetAsync(status, 0, (size_t)n * sizeof(int32_t), st));
-    if (launch(c, kind, a, o, user))
+    if (dispatch_kind(kind, [&](auto k) { return launch_kind<decltype(k)::value>(c, a, o, user); }))
         return 1;
     RB_CUDA(cudaEventRecord(c.ev_done, st));
     c.have_done = true;
@@ -451,17 +463,11 @@ int run_host(int kind, int64_t n, const double *s, const double *theta, const do
              int device_override, int64_t out_stride = 0)
 {
     DeviceGuard restore_device;
-    if (n < 0)
-        return fail("n_points is negative");
-    if (check_params(kind, n_params))
+    ResolvedOptions o;
+    if (check_batch(kind, n, s, theta, params, n_params, out8, opts, &o))
         return 1;
     if (n == 0)
         return 0;
-    if (!s || !theta || !params || !out8)
-        return fail("null array pointer");
-    ResolvedOptions o = resolve(opts);
-    if (o.mode < 0 || o.mode > 3)
-        return fail("unknown mode %d", o.mode);
     if (device_override >= 0)
         o.device = device_override;
 
@@ -579,17 +585,11 @@ int rimphony_b200_compute_all_dimensionless_device(int kind, int64_t n_points, c
                                                    const rimphony_b200_options *opts, double *out8, int32_t *status,
                                                    const rimphony_b200_extras *extras, void *stream, int synchronize)
 {
-    if (n_points < 0)
-        return fail("n_points is negative");
-    if (check_params(kind, n_params))
+    ResolvedOptions o;
+    if (check_batch(kind, n_points, s, theta, params, n_params, out8, opts, &o))
         return 1;
     if (n_points == 0)
         return 0;
-    if (!s || !theta || !params || !out8)
-        return fail("null array pointer");
-    ResolvedOptions o = resolve(opts);
-    if (o.mode < 0 || o.mode > 3)
-        return fail("unknown mode %d", o.mode);
     DeviceGuard restore_device;
     DeviceContext *cp = nullptr;
     if (get_context(o.device, &cp))
@@ -603,20 +603,14 @@ int rimphony_b200_compute_all_dimensionless_multi(int kind, int64_t n_points, co
                                                   const rimphony_b200_options *opts, double *out8, int32_t *status,
                                                   int n_devices)
 {
-    if (n_points < 0)
-        return fail("n_points is negative");
-    if (check_params(kind, n_params))
+    ResolvedOptions o;
+    if (check_batch(kind, n_points, s, theta, params, n_params, out8, opts, &o))
         return 1;
     if (n_points == 0)
         return 0;
-    if (!s || !theta || !params || !out8)
-        return fail("null array pointer");
     for (int j = 0; j < n_params; j++)
         if (!params[j])
             return fail("params[%d] is null", j);
-    const ResolvedOptions o = resolve(opts);
-    if (o.mode < 0 || o.mode > 3)
-        return fail("unknown mode %d", o.mode);
     int visible = 0;
     RB_CUDA(cudaGetDeviceCount(&visible));
     if (visible < 1)
@@ -766,22 +760,11 @@ int rimphony_b200_diagnostic_symphony(int kind, const double *params, int n_para
     ba.eps_gamma = ba.eps_n = 1e-3;
     DiagArgs g{coeff, stokes, what, (long long)count, d_a, b ? d_b : nullptr, d_out, d_status};
 
-    int rc;
-    switch (kind) {
-    case RIMPHONY_B200_POWER_LAW:
-        rc = diag_kind<kDistPowerLaw>(c, ba, g);
-        break;
-    case RIMPHONY_B200_THERMAL_JUETTNER:
-        rc = diag_kind<kDistThermalJuettner>(c, ba, g);
-        break;
-    case RIMPHONY_B200_PITCHY_PL:
-        rc = diag_kind<kDistPitchyPL>(c, ba, g);
-        break;
-    default:
-        rc = diag_kind<kDistPitchyKappa>(c, ba, g);
-        break;
-    }
-    if (rc)
+    if (dispatch_kind(kind, [&](auto k) {
+            constexpr int KIND = decltype(k)::value;
+            return stage_normalize<KIND>(ba, c.sm_count, c.stream) ||
+                   stage_symphony_diag<KIND>(ba, g, c.sm_count, c.stream);
+        }))
         return 1;
     RB_CUDA(cudaMemcpyAsync(out, d_out, (size_t)count * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
     if (status)
@@ -840,22 +823,9 @@ int rimphony_b200_dist_eval(int kind, const double *params, int n_params, int64_
     double *d_o = static_cast<double *>(c.out.ptr);
     RB_CUDA(cudaMemcpyAsync(d_g, gamma, bytes, cudaMemcpyHostToDevice, c.stream));
     RB_CUDA(cudaMemcpyAsync(d_c, cos_xi, bytes, cudaMemcpyHostToDevice, c.stream));
-    int rc;
-    switch (kind) {
-    case RIMPHONY_B200_POWER_LAW:
-        rc = stage_dist_eval<kDistPowerLaw>(params, n_params, count, d_g, d_c, d_o, c.stream);
-        break;
-    case RIMPHONY_B200_THERMAL_JUETTNER:
-        rc = stage_dist_eval<kDistThermalJuettner>(params, n_params, count, d_g, d_c, d_o, c.stream);
-        break;
-    case RIMPHONY_B200_PITCHY_PL:
-        rc = stage_dist_eval<kDistPitchyPL>(params, n_params, count, d_g, d_c, d_o, c.stream);
-        break;
-    default:
-        rc = stage_dist_eval<kDistPitchyKappa>(params, n_params, count, d_g, d_c, d_o, c.stream);
-        break;
-    }
-    if (rc)
+    if (dispatch_kind(kind, [&](auto k) {
+            return stage_dist_eval<decltype(k)::value>(params, n_params, count, d_g, d_c, d_o, c.stream);
+        }))
         return 1;
     RB_CUDA(cudaMemcpyAsync(out3, d_o, 3 * bytes, cudaMemcpyDeviceToHost, c.stream));
     RB_CUDA(cudaStreamSynchronize(c.stream));

@@ -1,6 +1,7 @@
-"""Kernel-tuning A/B on the GPU box: one build of the library (RIMPHONY_B200_LIB selects a variant from
-rimphony_b200/variants/, see csrc/Makefile `variant`) on the seeded pitchy power-law batch; prints kernel
-times and a checksum of the results (variants that only change scheduling must reproduce it bit for bit).
+"""A/B of two builds of the library: runs the one RIMPHONY_B200_LIB names (default: the in-tree build; another
+one comes from `make -C rimphony_b200/csrc OUT=... OBJDIR=...` in a second checkout) on the seeded pitchy
+power-law batch and prints kernel times and a digest of the results (builds that only change scheduling or
+code layout must reproduce it bit for bit).
 usage: [RIMPHONY_B200_LIB=...] python tools/variant_bench.py [N=131072] [CONFIG=pitchy_pl] [REPS=2]"""
 import hashlib
 import os
