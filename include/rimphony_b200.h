@@ -39,13 +39,18 @@ extern "C" {
  *   THERMAL_JUETTNER  T                                                1 column
  *   PITCHY_PL         p, k [, gamma_min, gamma_max, gamma_cutoff]     2 or 5 columns
  *   PITCHY_KAPPA      kappa, width, k [, gamma_cutoff]                 3 or 4 columns
+ *   PITCHY_BROKEN_PL  p1, p2, gamma_break, k                           4 or 7 columns
+ *                     [, gamma_min, gamma_max, gamma_cutoff]
+ *                     gamma^-p1 below gamma_break, gamma_break^(p2 - p1) gamma^-p2 from it on,
+ *                     times sin^k(xi) as in PITCHY_PL
  * Omitted trailing columns take the reference's defaults: gamma_min = 1,
  * gamma_max = 1e12, gamma_cutoff = 1e10. */
 enum rimphony_b200_dist_kind {
     RIMPHONY_B200_POWER_LAW = 0,
     RIMPHONY_B200_THERMAL_JUETTNER = 1,
     RIMPHONY_B200_PITCHY_PL = 2,
-    RIMPHONY_B200_PITCHY_KAPPA = 3
+    RIMPHONY_B200_PITCHY_KAPPA = 3,
+    RIMPHONY_B200_PITCHY_BROKEN_PL = 4
 };
 
 /* src/lib.rs:92-107 and :75-87 */

@@ -9,6 +9,8 @@ Host-side mirror of the reference's public interface for this path (pkgw/rimphon
 * ``ThermalJuettnerDistribution(t)``                src/thermal_juettner.rs:45-50
 * ``PitchyPowerLawDistribution(p, k).gamma_limits(..)``  src/pitchy_pl.rs:73-90
 * ``PitchyKappaDistribution(kappa, width, k).gamma_cutoff(..)``  src/pitchy_kappa.rs:70-85
+* ``PitchyBrokenPowerLawDistribution(p1, p2, gamma_break, k).gamma_limits(..)``  a broken power law
+  built as src/pitchy_pl.rs builds its single one (no counterpart in the reference)
 * ``.full_calculation(logger)`` -> ``FullSynchrotronCalculator`` with the trait
   methods ``compute_dimensionless``, ``compute_cgs``, ``compute_all_dimensionless``,
   ``compute_all_cgs``                               src/lib.rs:150-247
@@ -38,7 +40,7 @@ MASS_ELECTRON = 9.1093826e-28
 SPEED_LIGHT = 2.99792458e10
 ELECTRON_CHARGE = 4.80320680e-10
 
-POWER_LAW, THERMAL_JUETTNER, PITCHY_PL, PITCHY_KAPPA = 0, 1, 2, 3
+POWER_LAW, THERMAL_JUETTNER, PITCHY_PL, PITCHY_KAPPA, PITCHY_BROKEN_PL = 0, 1, 2, 3, 4
 
 MODE_FAST, MODE_FAITHFUL, MODE_FUSED_ALL, MODE_FUSED = 0, 1, 2, 3
 
@@ -509,6 +511,25 @@ class PitchyPowerLawDistribution(_Distribution):
 
     def _columns(self):
         return [self.p, self.k, self.gamma_min, self.gamma_max, self._gamma_cutoff]
+
+
+class PitchyBrokenPowerLawDistribution(_Distribution):
+    """A broken power law times sin^k(pitch angle), built as src/pitchy_pl.rs builds its single one:
+    dN/dgamma ~ gamma^-p1 below gamma_break and gamma_break^(p2 - p1) gamma^-p2 from it on (continuous
+    at the break), times exp(-gamma/gamma_cutoff), on [gamma_min, gamma_max].  p1 = p2, or a break at
+    or above gamma_max, is PitchyPowerLawDistribution(p1, k)."""
+    KIND = PITCHY_BROKEN_PL
+
+    def __init__(self, p1, p2, gamma_break, k):
+        self.p1, self.p2, self.gamma_break, self.k = p1, p2, gamma_break, k
+        self.gamma_min, self.gamma_max, self._gamma_cutoff = 1.0, 1e12, 1e10
+
+    def gamma_limits(self, gamma_min, gamma_max, gamma_cutoff):
+        self.gamma_min, self.gamma_max, self._gamma_cutoff = gamma_min, gamma_max, gamma_cutoff
+        return self
+
+    def _columns(self):
+        return [self.p1, self.p2, self.gamma_break, self.k, self.gamma_min, self.gamma_max, self._gamma_cutoff]
 
 
 class PitchyKappaDistribution(_Distribution):

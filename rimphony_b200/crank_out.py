@@ -4,6 +4,8 @@
     python -m rimphony_b200.crank_out pitchypl   S_MIN S_MAX THETA_MIN THETA_MAX P_MIN P_MAX K_MIN K_MAX OUTFILE
     python -m rimphony_b200.crank_out pitchykappa S_MIN S_MAX THETA_MIN THETA_MAX KAPPA_MIN KAPPA_MAX \\
                                                   WIDTH_MIN WIDTH_MAX K_MIN K_MAX OUTFILE
+    python -m rimphony_b200.crank_out pitchybpl   S_MIN S_MAX THETA_MIN THETA_MAX P1_MIN P1_MAX P2_MIN P2_MAX \
+                                                  GAMMA_BREAK_MIN GAMMA_BREAK_MAX K_MIN K_MAX OUTFILE
     python -m rimphony_b200.crank_out demo almostuniform1          # examples/demo-powerlaw.rs, to stdout
 
 Same positional arguments (crank-out-pitchypl.rs:17-74, crank-out-pitchykappa.rs:17-92), same
@@ -15,6 +17,10 @@ blocks of ``--block`` points, evaluates each block with one batched call and app
 ``time_ms(meta)`` is the block's wall time divided by the block size.  ``--count`` stops after
 that many points (default: run until interrupted, like the reference); ``--gpus`` shards each
 block over several GPUs of the box.
+
+``pitchybpl`` has no counterpart in the reference: it is ``pitchypl`` for the pitchy broken power law
+(``PitchyBrokenPowerLawDistribution``), with gamma_break drawn log-uniform and p1, p2 uniform, each
+from its own range.
 """
 import argparse
 import sys
@@ -28,6 +34,10 @@ PITCHYPL_HEADER = ("s(log)", "theta(lin)", "p(lin)", "k(lin)", "time_ms(meta)", 
                    "alpha_Q(res)", "j_V(res)", "alpha_V(res)", "rho_Q(res)", "rho_V(res)")
 PITCHYKAPPA_HEADER = ("s(log)", "theta(lin)", "kappa(lin)", "width(log)", "k(lin)", "time_ms(meta)", "j_I(res)",
                       "alpha_I(res)", "j_Q(res)", "alpha_Q(res)", "j_V(res)", "alpha_V(res)", "rho_Q(res)", "rho_V(res)")
+
+PITCHYBPL_HEADER = ("s(log)", "theta(lin)", "p1(lin)", "p2(lin)", "gamma_break(log)", "k(lin)", "time_ms(meta)",
+                    "j_I(res)", "alpha_I(res)", "j_Q(res)", "alpha_Q(res)", "j_V(res)", "alpha_V(res)", "rho_Q(res)",
+                    "rho_V(res)")
 
 DEMO_HEADER = ("s(lin)", "theta(lin)", "p(lin)", "d(meta)", "psi(meta)", "n_e(meta)", "time_ms(meta)", "j_I(res)",
                "alpha_I(res)", "j_Q(res)", "alpha_Q(res)", "j_V(res)", "alpha_V(res)", "rho_Q(res)", "rho_V(res)")
@@ -96,6 +106,11 @@ def parse(argv):
                  "K_MIN", "K_MAX"):
         pk.add_argument(name, type=float)
     pk.add_argument("OUTFILE")
+    pb = sub.add_parser("pitchybpl")
+    for name in ("S_MIN", "S_MAX", "THETA_MIN", "THETA_MAX", "P1_MIN", "P1_MAX", "P2_MIN", "P2_MAX", "GAMMA_BREAK_MIN",
+                 "GAMMA_BREAK_MAX", "K_MIN", "K_MAX"):
+        pb.add_argument(name, type=float)
+    pb.add_argument("OUTFILE")
     dm = sub.add_parser("demo")
     dm.add_argument("DEMONAME", choices=["almostuniform1"])
     return ap.parse_args(argv)
@@ -108,6 +123,13 @@ def samplers(args, rng):
                                  ("theta", Sampler(False, args.THETA_MIN, args.THETA_MAX, rng)),
                                  ("p", Sampler(False, args.P_MIN, args.P_MAX, rng)),
                                  ("k", Sampler(False, args.K_MIN, args.K_MAX, rng))]
+    if args.tool == "pitchybpl":
+        return PITCHYBPL_HEADER, [("s", Sampler(True, args.S_MIN, args.S_MAX, rng)),
+                                  ("theta", Sampler(False, args.THETA_MIN, args.THETA_MAX, rng)),
+                                  ("p1", Sampler(False, args.P1_MIN, args.P1_MAX, rng)),
+                                  ("p2", Sampler(False, args.P2_MIN, args.P2_MAX, rng)),
+                                  ("gamma_break", Sampler(True, args.GAMMA_BREAK_MIN, args.GAMMA_BREAK_MAX, rng)),
+                                  ("k", Sampler(False, args.K_MIN, args.K_MAX, rng))]
     return PITCHYKAPPA_HEADER, [("s", Sampler(True, args.S_MIN, args.S_MAX, rng)),
                                 ("theta", Sampler(False, args.THETA_MIN, args.THETA_MAX, rng)),
                                 ("kappa", Sampler(False, args.KAPPA_MIN, args.KAPPA_MAX, rng)),
@@ -121,6 +143,9 @@ def evaluate(tool, cols, n_devices):
 
     if tool == "pitchypl":
         kind, params = R.PITCHY_PL, [cols["p"], cols["k"], GAMMA_MIN, GAMMA_MAX, GAMMA_CUTOFF]
+    elif tool == "pitchybpl":
+        kind, params = R.PITCHY_BROKEN_PL, [cols["p1"], cols["p2"], cols["gamma_break"], cols["k"], GAMMA_MIN, GAMMA_MAX,
+                                            GAMMA_CUTOFF]
     else:
         kind, params = R.PITCHY_KAPPA, [cols["kappa"], cols["width"], cols["k"], GAMMA_CUTOFF]
     res = R.compute_all_dimensionless_batch(kind, cols["s"], cols["theta"], params,

@@ -1,11 +1,12 @@
-// rb_dist.cuh -- the four electron distribution functions and their
-// normalisation ("full_calculation") as device code.
+// rb_dist.cuh -- the electron distribution functions and their normalisation
+// ("full_calculation") as device code.
 //
 // Replaces (reference file:line):
 //   src/power_law.rs:36-62, 93-103         PowerLawDistribution
 //   src/thermal_juettner.rs:29-39, 56-64   ThermalJuettnerDistribution
 //   src/pitchy_pl.rs:32-64, 95-115         PitchyPowerLawDistribution
 //   src/pitchy_kappa.rs:38-62, 90-125      PitchyKappaDistribution
+// and a pitchy broken power law built the way src/pitchy_pl.rs builds its single one.
 //
 // f, df/dgamma and df/dcos(xi) are produced together: they share one rb_exp() and
 // one or two rb_log() per call (gamma^-p rb_exp(-gamma/gc) sin^k(xi) is evaluated as a
@@ -17,15 +18,21 @@
 namespace rb {
 
 // numbering shared with include/rimphony_b200.h
-enum { kDistPowerLaw = 0, kDistThermalJuettner = 1, kDistPitchyPL = 2, kDistPitchyKappa = 3 };
+enum { kDistPowerLaw = 0, kDistThermalJuettner = 1, kDistPitchyPL = 2, kDistPitchyKappa = 3, kDistPitchyBrokenPL = 4 };
 
 struct Dist {
-    double p, k;
+    double p, k; // p: the index below the break for PITCHY_BROKEN_PL
     double gamma_min, gamma_max, inv_gamma_cutoff;
     double kappa, width, inv_kappa_width;
     double neg_inverse_t;
     double norm;
 };
+
+// PITCHY_BROKEN_PL keeps p2, gamma_break and (p2 - p1) ln(gamma_break) in the kappa fields, which it does not
+// use.  (Named fields in a union there would change how the other kinds' kernels compile.)
+RB_HD double bpl_p2(const Dist &d) { return d.kappa; }
+RB_HD double bpl_gamma_break(const Dist &d) { return d.width; }
+RB_HD double bpl_log_offset(const Dist &d) { return d.inv_kappa_width; }
 
 // Fill `d` from the C-ABI parameter vector of one point (see the header for
 // the order); `norm` is left NaN until dist_normalize<>() has run.
@@ -59,6 +66,19 @@ RB_HD bool dist_from_params(const double *pv, int n_params, Dist &d)
             d.gamma_min = pv[2];
             d.gamma_max = pv[3];
             d.inv_gamma_cutoff = 1.0 / pv[4];
+        }
+    } else if (KIND == kDistPitchyBrokenPL) {
+        if (n_params != 4 && n_params != 7)
+            return false;
+        d.p = pv[0];
+        d.kappa = pv[1];                          // bpl_p2
+        d.width = pv[2];                          // bpl_gamma_break
+        d.inv_kappa_width = (pv[1] - pv[0]) * log(pv[2]); // bpl_log_offset
+        d.k = pv[3];
+        if (n_params == 7) {
+            d.gamma_min = pv[4];
+            d.gamma_max = pv[5];
+            d.inv_gamma_cutoff = 1.0 / pv[6];
         }
     } else {
         if (n_params != 3 && n_params != 4)
@@ -117,6 +137,25 @@ RB_FN void dist_eval(const Dist &d, double gamma, double cos_xi, double &f, doub
         f = d.norm * rb_exp(log_pitch_term(d.k, sin2) - d.p * rb_log(gamma) - gamma * d.inv_gamma_cutoff) * inv;
         dfdg = -f * ((d.p + 1.0) * (inv * sq) + gamma * (ig * ig) + d.inv_gamma_cutoff);
         dfdcx = -f * d.k * rb_div(cos_xi, sin2);
+    } else if (KIND == kDistPitchyBrokenPL) {
+        if (gamma < d.gamma_min || gamma > d.gamma_max) {
+            f = dfdg = dfdcx = 0.0;
+            return;
+        }
+        // PITCHY_PL with gamma^-p1 below the break and gamma_break^(p2 - p1) gamma^-p2 from it on
+        const bool upper = !(gamma < bpl_gamma_break(d));
+        const double p = upper ? bpl_p2(d) : d.p;
+        const double sin2 = (sin2_exact == sin2_exact) ? sin2_exact : 1.0 - cos_xi * cos_xi;
+        const double g2m1 = gamma * gamma - 1.0;
+        const double sq = (sqrt_g2m1 == sqrt_g2m1) ? sqrt_g2m1 : rb_sqrt(g2m1);
+        const double inv = rb_rcp(gamma * sq);
+        const double ig = inv * gamma;
+        f = d.norm *
+            rb_exp(log_pitch_term(d.k, sin2) + (upper ? bpl_log_offset(d) : 0.0) - p * rb_log(gamma) -
+                   gamma * d.inv_gamma_cutoff) *
+            inv;
+        dfdg = -f * ((p + 1.0) * (inv * sq) + gamma * (ig * ig) + d.inv_gamma_cutoff);
+        dfdcx = -f * d.k * rb_div(cos_xi, sin2);
     } else {
         const double sin2 = (sin2_exact == sin2_exact) ? sin2_exact : 1.0 - cos_xi * cos_xi;
         f = d.norm * rb_exp(log_pitch_term(d.k, sin2) -
@@ -132,6 +171,15 @@ RB_FN void dist_eval(const Dist &d, double gamma, double cos_xi, double &f, doub
 struct PLNormIntegrand {
     double p, inv_gamma_cutoff;
     RB_FN void eval(double g, double (&out)[1]) const { out[0] = rb_exp(-p * rb_log(g) - g * inv_gamma_cutoff); }
+};
+
+struct BrokenPLNormIntegrand {
+    double p1, p2, gamma_break, log_offset, inv_gamma_cutoff;
+    RB_FN void eval(double g, double (&out)[1]) const
+    {
+        const bool upper = !(g < gamma_break);
+        out[0] = rb_exp((upper ? log_offset : 0.0) - (upper ? p2 : p1) * rb_log(g) - g * inv_gamma_cutoff);
+    }
 };
 
 struct KappaNormIntegrand {
@@ -203,6 +251,14 @@ RB_FN bool dist_normalize(Warp &w, Dist &d, double t_juettner, IntervalList<1> &
         qag_joint<PolicyPlain<1>>(w, ap, 1, bounds, 1e-8, list, 1u, integral);
         if (KIND == kDistPitchyPL)
             pa = pitch_angle_integral(d.k);
+    } else if (KIND == kDistPitchyBrokenPL) {
+        // one QAG over the whole range, no split at the break: what the reference's
+        // full_calculation (pitchy_pl.rs:95-112) does with this gamma term
+        BrokenPLNormIntegrand f{d.p, bpl_p2(d), bpl_gamma_break(d), bpl_log_offset(d), d.inv_gamma_cutoff};
+        ApplyLanes<1, BrokenPLNormIntegrand> ap{f};
+        const double bounds[2] = {d.gamma_min, d.gamma_max};
+        qag_joint<PolicyPlain<1>>(w, ap, 1, bounds, 1e-8, list, 1u, integral);
+        pa = pitch_angle_integral(d.k);
     } else {
         KappaNormIntegrand f{d.kappa, d.inv_kappa_width, d.inv_gamma_cutoff};
         ApplyLanes<1, KappaNormIntegrand> ap{f};

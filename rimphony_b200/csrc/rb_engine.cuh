@@ -482,6 +482,58 @@ struct PanelStack {
         b = store.stk_b[sp];
         tag = store.stk_tag[sp];
     }
+
+    // Cut the pending panel that straddles t at t, in its place in the stack (the pending panels are
+    // disjoint): where the integrand jumps at t, no rule is then applied across the jump.  `paired`:
+    // the panels are popped two at a time, so the pop partner is cut at the same fraction of its width
+    // and each pop pair holds one part of both: a pair then still lies inside the pair it was cut from
+    // (for the gamma integral: inside one Bessel branch).  A NaN t, or no room, cuts nothing.  Call
+    // between the pushes and seal().
+    RB_FN void cut_at(const Warp &w, double t, bool paired)
+    {
+        warp_fence(); // lane 0's pushes
+        int i = -1;
+        for (int j = 0; j < sp; j++) {
+            if (store.stk_a[j] < t && t < store.stk_b[j])
+                i = j;
+        }
+        // pop pairs run from the top, (sp - 1, sp - 2), ...; a bottom panel left over is popped alone
+        const bool pair = paired && !(i == 0 && (sp & 1));
+        const int lo = pair ? i - ((sp - 1 - i) & 1 ? 0 : 1) : i; // first entry of the pair
+        const int grow = pair ? 2 : 1;
+        if (i < 0 || !room(grow))
+            return;
+        warp_fence(); // every lane has read the stack
+#ifdef RB_DEVICE_BUILD
+        if (w.lane == 0)
+#endif
+        {
+            for (int j = sp - 1; j > i; j--) { // the entries above make room
+                store.stk_a[j + grow] = store.stk_a[j];
+                store.stk_b[j + grow] = store.stk_b[j];
+                store.stk_tag[j + grow] = store.stk_tag[j];
+            }
+            if (pair) { // [a0, c0], [a1, c1] below [c0, b0], [c1, b1]
+                const double frac = (t - store.stk_a[i]) / (store.stk_b[i] - store.stk_a[i]);
+                for (int k = 1; k >= 0; k--) {
+                    const double a = store.stk_a[lo + k], b = store.stk_b[lo + k];
+                    const int tag = store.stk_tag[lo + k];
+                    const double c = (lo + k == i) ? t : a + frac * (b - a);
+                    store.stk_a[lo + k] = a;
+                    store.stk_b[lo + k] = c;
+                    store.stk_a[lo + 2 + k] = c;
+                    store.stk_b[lo + 2 + k] = b;
+                    store.stk_tag[lo + 2 + k] = tag;
+                }
+            } else { // [t, b] below [a, t]: the lower part is popped first
+                store.stk_a[i + 1] = store.stk_a[i];
+                store.stk_b[i + 1] = t;
+                store.stk_tag[i + 1] = store.stk_tag[i];
+                store.stk_a[i] = t;
+            }
+        }
+        sp += grow;
+    }
 };
 
 // The acceptance rule of a panel for one channel: the error estimate is within

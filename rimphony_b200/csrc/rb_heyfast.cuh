@@ -145,6 +145,12 @@ RB_FN_NOINLINE bool hey_inner_integral(Warp &w, const HeyFastCtx<KIND> &cx, int 
             n_seed = n_seed < 1 ? 1 : (n_seed > 8 ? 8 : n_seed);
             for (int k = n_seed - 1; k >= 0; k--) // the lowest panel (largest values) is popped first
                 stk.push(w, t_lo + (t_hi - t_lo) * k / n_seed, (k + 1 == n_seed) ? t_hi : t_lo + (t_hi - t_lo) * (k + 1) / n_seed, 0);
+            if (KIND == kDistPitchyBrokenPL) {
+                // df/dsigma jumps where the line gamma = gamma_break, sigma = gamma_break sigma0 sin(theta) +
+                // pomega cos(theta), crosses the range: cut at its t
+                const double r = (bpl_gamma_break(*cx.d) * g.sigma0 * g.sin_th + v * g.cos_th) / sigma_min;
+                stk.cut_at(w, (r > 1.0) ? rb_log(r + rb_sqrt((r - 1.0) * (r + 1.0))) : NAN, false);
+            }
         }
     } else {
         // heyvaerts.rs:262-296: pomega in [-pomega_max, pomega_max]
@@ -217,6 +223,12 @@ RB_FN_NOINLINE bool hey_inner_integral(Warp &w, const HeyFastCtx<KIND> &cx, int 
                 stk.push(w, -cut, cut, 0);
             } else
                 stk.push(w, -end, end, 0);
+            if (KIND == kDistPitchyBrokenPL) {
+                // df/dsigma jumps on the line gamma = gamma_break, pomega = (sigma - gamma_break sigma0 sin(theta)) /
+                // cos(theta): cut at its pomega, or its phi under the sine map (NaN outside the range: no cut)
+                const double pomega_b = (v - bpl_gamma_break(*cx.d) * g.sigma0 * g.sin_th) / g.cos_th;
+                stk.cut_at(w, sine_map ? asin(pomega_b / sine_amp) : pomega_b, false);
+            }
         }
     }
     stk.seal();
@@ -604,7 +616,9 @@ RB_FN void heyvaerts_point_fast(Warp &w, const Dist &dist, double s, double thet
     RB_FOR_CHAN(c, 2) { alive[c] = true; }
     const double div_q = hey_ref_diverges_q(KIND == kDistPowerLaw, cx.g.sin_th, cx.g.cos_th);
     const double div_v = (KIND == kDistPowerLaw) ? kHeyRefDivergesIsoV : kHeyRefDivergesV;
-    if ((KIND == kDistPowerLaw || KIND == kDistPitchyPL) && dist.gamma_min == 1.0 && s < div_v) {
+    // (the broken power law is PITCHY_PL with p = p1 near gamma = 1: the same rule, the same thresholds)
+    if ((KIND == kDistPowerLaw || KIND == kDistPitchyPL || KIND == kDistPitchyBrokenPL) && dist.gamma_min == 1.0 &&
+        s < div_v) {
         // the reference's NaN region (see kHeyRefDivergesQ)
         w.status |= kStatusRefDiverges;
         RB_FOR_CHAN(c, 2) { alive[c] = (c == 0) && !(s < div_q); }

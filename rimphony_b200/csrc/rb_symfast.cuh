@@ -435,6 +435,9 @@ RB_FN_NOINLINE void sym_gamma_integral(Warp &w, const SymFastCtx<KIND> &cx, doub
                 stk.push(w, side ? lo : -hi, side ? hi : -lo, side);
         }
     }
+    // A broken power law's df/dgamma jumps at the break, and f has a kink there: no panel straddles it.
+    if (KIND == kDistPitchyBrokenPL)
+        stk.cut_at(w, (bpl_gamma_break(*cx.d) - gamma_peak) / half, true);
     stk.seal();
 
     // Every application carries TWO panels as 15-point Kronrod rules, one per half warp (lanes

@@ -254,6 +254,9 @@ int check_params(int kind, int n_params)
         return (n_params == 2 || n_params == 5) ? 0 : fail("PITCHY_PL takes 2 or 5 parameter columns, got %d", n_params);
     case RIMPHONY_B200_PITCHY_KAPPA:
         return (n_params == 3 || n_params == 4) ? 0 : fail("PITCHY_KAPPA takes 3 or 4 parameter columns, got %d", n_params);
+    case RIMPHONY_B200_PITCHY_BROKEN_PL:
+        return (n_params == 4 || n_params == 7) ? 0
+                                                : fail("PITCHY_BROKEN_PL takes 4 or 7 parameter columns, got %d", n_params);
     }
     return fail("unknown distribution kind %d", kind);
 }
@@ -291,7 +294,9 @@ int launch_kind(DeviceContext &c, BatchArgs a, const ResolvedOptions &o, cudaStr
 
     RB_CUDA(cudaMemsetAsync(counters, 0, 4 * sizeof(unsigned long long), st));
     RB_CUDA(cudaEventRecord(c.ev[0], st));
-    a.hey_free_below = (KIND == kDistPitchyPL) ? kHeyDivQLo : ((KIND == kDistPowerLaw) ? 0.05 : 0.0);
+    // the broken power law is PITCHY_PL with p = p1 near gamma = 1, where the reference diverges
+    a.hey_free_below =
+        (KIND == kDistPitchyPL || KIND == kDistPitchyBrokenPL) ? kHeyDivQLo : ((KIND == kDistPowerLaw) ? 0.05 : 0.0);
 
     // 1. normalisation (+ the cost-ordered schedule of the product kernels)
     if (stage_normalize<KIND>(a, c.sm_count, st))
@@ -367,6 +372,8 @@ int dispatch_kind(int kind, F &&f)
         return f(std::integral_constant<int, kDistPitchyPL>{});
     case RIMPHONY_B200_PITCHY_KAPPA:
         return f(std::integral_constant<int, kDistPitchyKappa>{});
+    case RIMPHONY_B200_PITCHY_BROKEN_PL:
+        return f(std::integral_constant<int, kDistPitchyBrokenPL>{});
     }
     return fail("unknown distribution kind %d", kind);
 }

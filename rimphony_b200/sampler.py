@@ -9,7 +9,7 @@ import math
 
 import numpy as np
 
-POWER_LAW, THERMAL_JUETTNER, PITCHY_PL, PITCHY_KAPPA = 0, 1, 2, 3
+POWER_LAW, THERMAL_JUETTNER, PITCHY_PL, PITCHY_KAPPA, PITCHY_BROKEN_PL = 0, 1, 2, 3, 4
 
 
 class Sampler:
@@ -47,6 +47,12 @@ CONFIGS = {
                      [("s", True, 1.0, 1e6), ("theta", False, 0.003, 1.5705), ("kappa", False, 1.5, 4.5),
                       ("width", True, math.e, math.e ** 3), ("k", False, 0.0, 3.0)],
                      [1e10]),
+    # a cooled population: a power law that steepens by 0.5-1.5 above a break; the drawn column
+    # `dp` is replaced by p2 = p1 + dp
+    "pitchy_bpl": (PITCHY_BROKEN_PL,
+                   [("s", True, 0.07, 1e4), ("theta", False, 0.003, 1.5705), ("p1", False, 1.5, 3.0),
+                    ("dp", False, 0.5, 1.5), ("gamma_break", True, 10.0, 1e4), ("k", False, 0.0, 3.0)],
+                   [1.0, 1e12, 1e10]),
 }
 
 
@@ -70,6 +76,8 @@ def synthetic_batch(config, n, seed=20260, shard=0, sequential=False):
         if not sequential:
             rng = np.random.Generator(np.random.Philox(key=[int(seed), int(shard)], counter=[0, 0, 0, j + 1]))
         drawn[name] = Sampler(is_log, lo, hi, rng).get(n)
+    if "dp" in drawn:
+        drawn["dp"] = drawn["p1"] + drawn["dp"]
     s = drawn.pop("s")
     theta = drawn.pop("theta")
     params = [drawn[name] for name, *_ in cols[2:]] + list(fixed)

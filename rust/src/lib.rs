@@ -1,6 +1,6 @@
 //! Rust facade over `include/rimphony_b200.h`.
 //!
-//! Keeps the reference's public surface for the hot path -- `Coefficient`, `Stokes`, the four
+//! Keeps the reference's public surface for the hot path -- `Coefficient`, `Stokes`, the
 //! distribution types with their builders, `full_calculation()`, and the
 //! `SynchrotronCalculator` trait (reference `src/lib.rs:75-107, 150-210, 231-247`) -- and adds the
 //! batched call the GPU path is built for.  Numerical failure is `NaN`, never a panic or an
@@ -147,6 +147,41 @@ impl B200Params for PitchyPowerLawDistribution {
     const KIND: c_int = 2;
     fn b200_params(&self) -> Vec<f64> {
         vec![self.p, self.k, self.gamma_min, self.gamma_max, self.gamma_cutoff]
+    }
+}
+
+/// A broken power law times sin^k(pitch angle): gamma^-p1 below `gamma_break`,
+/// gamma_break^(p2 - p1) gamma^-p2 from it on, built as src/pitchy_pl.rs:22-90 builds its single one.
+#[derive(Copy, Clone, Debug, PartialEq)]
+pub struct PitchyBrokenPowerLawDistribution {
+    p1: f64,
+    p2: f64,
+    gamma_break: f64,
+    k: f64,
+    gamma_min: f64,
+    gamma_max: f64,
+    gamma_cutoff: f64,
+}
+
+impl PitchyBrokenPowerLawDistribution {
+    pub fn new(p1: f64, p2: f64, gamma_break: f64, k: f64) -> Self {
+        PitchyBrokenPowerLawDistribution { p1, p2, gamma_break, k, gamma_min: 1., gamma_max: 1e12, gamma_cutoff: 1e10 }
+    }
+    pub fn gamma_limits(mut self, gamma_min: f64, gamma_max: f64, gamma_cutoff: f64) -> Self {
+        self.gamma_min = gamma_min;
+        self.gamma_max = gamma_max;
+        self.gamma_cutoff = gamma_cutoff;
+        self
+    }
+    pub fn full_calculation<L>(self, _logger: L) -> FullSynchrotronCalculator<Self> {
+        FullSynchrotronCalculator::new(self)
+    }
+}
+
+impl B200Params for PitchyBrokenPowerLawDistribution {
+    const KIND: c_int = 4;
+    fn b200_params(&self) -> Vec<f64> {
+        vec![self.p1, self.p2, self.gamma_break, self.k, self.gamma_min, self.gamma_max, self.gamma_cutoff]
     }
 }
 
