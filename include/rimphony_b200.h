@@ -212,6 +212,66 @@ int rimphony_b200_bessel_jn(int64_t count, const double *n, const double *x, dou
 int rimphony_b200_dist_eval(int kind, const double *params, int n_params, int64_t count, const double *gamma,
                             const double *cos_xi, double *out3);
 
+/* Polarized radiative transfer through rays of cells (DESIGN.md section 13).
+ *
+ * In each cell the eight coefficients are constant, in the units of compute_all_cgs (j in
+ * erg s^-1 cm^-3 Hz^-1 sr^-1, alpha and rho in cm^-1), and along the path s
+ *
+ *     dS/ds = J - K S,   S = (I, Q, U, V),   J = (j_I, j_Q c, j_Q s2, j_V)
+ *
+ *     K = | alpha_I      alpha_Q c    alpha_Q s2   alpha_V    |
+ *         | alpha_Q c    alpha_I      rho_V       -rho_Q s2   |
+ *         | alpha_Q s2  -rho_V        alpha_I      rho_Q c    |
+ *         | alpha_V      rho_Q s2    -rho_Q c      alpha_I    |
+ *
+ * with c = cos 2 psi and s2 = sin 2 psi: psi rotates the coefficients' frame, in which the U
+ * components are zero, into the observer's Stokes basis.  So with psi = 0, rho_V alone turns
+ * (Q, U) through +rho_V ds (Q -> U), and rho_Q alone turns (U, V) through +rho_Q ds (U -> V).
+ * Another convention maps onto this one by negating inputs: the sign of V (negate j_V, alpha_V and
+ * rho_V), the sense of the Faraday rotation (rho_V) or of psi.
+ *
+ * A ray has n_cells cells; cell 0 is where it enters, with the incident Stokes vector stokes0
+ * (zero if NULL), and cell n_cells - 1 is on the observer's side.  Each cell of length ds applies
+ *     S <- P S + Q J,   P = exp(-K ds),   Q = int_0^ds exp(-K t) dt,
+ * evaluated in closed form in FP64 (accurate for optically thin and thick cells up to alpha_I ds =
+ * 1e100, fully polarized absorption and Faraday depths |rho| ds up to 1e6).  A uniform slab is
+ * n_cells = 1.  Negative absorption (a masing cell) is supported down to alpha_I ds = -10; a cell
+ * with alpha_I ds below -10, or with alpha_I ds, |alpha_pol| ds or |rho| ds above 1e102, makes its
+ * ray NaN (split such a cell into shorter ones).
+ *
+ *   coeffs8   [8][n_rays * n_cells], slot-major in the order of out8; point index ray * n_cells + cell
+ *   psi, ds   [n_rays * n_cells] (radian, cm)
+ *   stokes0   [4][n_rays] or NULL
+ *   stokes4   [4][n_rays], the emergent (I, Q, U, V)
+ *   status    [n_rays] or NULL: RIMPHONY_B200_STATUS_NAN if the ray's Stokes vector is NaN, which it
+ *             is when an input of the ray is not finite, a ds is negative or a cell is out of range
+ * Host arrays.  Runs on the calling thread's current device. */
+int rimphony_b200_transfer(int64_t n_rays, int64_t n_cells, const double *coeffs8, const double *psi, const double *ds,
+                           const double *stokes0, double *stokes4, int32_t *status);
+
+/* Same, with every array a DEVICE pointer on the calling thread's current device and `stream` a
+ * cudaStream_t passed as void* (NULL = the library's own stream), as in
+ * rimphony_b200_compute_all_dimensionless_device.  Uses no scratch memory of the library. */
+int rimphony_b200_transfer_device(int64_t n_rays, int64_t n_cells, const double *coeffs8, const double *psi,
+                                  const double *ds, const double *stokes0, double *stokes4, int32_t *status,
+                                  void *stream, int synchronize);
+
+/* The whole chain for rays of cells, in one call on the device: s = nu / nu_c(b) per cell, the
+ * eight coefficients (opts as in the batched call; coeff_mask must be 0 or 0xFF), the cgs scaling of
+ * compute_all_cgs (src/lib.rs:196-209, the same operations in the same order, so both agree to the
+ * bit), then the transfer above with no incident radiation.
+ *   nu, b, n_e, theta, psi, ds   [n_rays * n_cells] (Hz, G, cm^-3, radian, radian, cm)
+ *   params       as in the batched call, [n_rays * n_cells] columns (or broadcast)
+ *   stokes4      [4][n_rays]
+ *   coeffs8_cgs  [8][n_rays * n_cells] or NULL: the cells' cgs coefficients
+ *   status       [n_rays] or NULL: the OR of the status words of the ray's cells, with
+ *                RIMPHONY_B200_STATUS_NAN set if the ray's Stokes vector is NaN
+ * Host arrays. */
+int rimphony_b200_compute_stokes_cgs(int kind, int64_t n_rays, int64_t n_cells, const double *nu, const double *b,
+                                     const double *n_e, const double *theta, const double *psi, const double *ds,
+                                     const double *const *params, int n_params, const rimphony_b200_options *opts,
+                                     double *stokes4, double *coeffs8_cgs, int32_t *status);
+
 /* Device time (ms, CUDA events on the launching stream) of the kernels of the most
  * recent batched call made by this thread's device: [0] normalisation,
  * [1] Symphony, [2] Heyvaerts, [3] whole enqueue-to-completion span. */

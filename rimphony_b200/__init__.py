@@ -15,6 +15,11 @@ Host-side mirror of the reference's public interface for this path (pkgw/rimphon
   methods ``compute_dimensionless``, ``compute_cgs``, ``compute_all_dimensionless``,
   ``compute_all_cgs``                               src/lib.rs:150-247
 
+Beyond the reference: ``transfer`` / ``transfer_device`` solve the polarized transfer equation
+through rays of cells with the eight cgs coefficients, and
+``FullSynchrotronCalculator.compute_stokes_cgs`` runs coefficients and transfer in one call
+(the convention is in ``include/rimphony_b200.h`` and DESIGN.md section 13).
+
 Same names, argument order and error behaviour (numerical failure = NaN in the
 slot, never an exception).  What is new is that every distribution parameter,
 ``s`` and ``theta`` may be arrays: one call then evaluates a whole batch of
@@ -247,6 +252,127 @@ def dist_eval(kind, params, gamma, cos_xi):
 
 
 # ---------------------------------------------------------------------------
+# Polarized transfer through rays of cells (include/rimphony_b200.h, DESIGN.md section 13).
+
+
+def _ray_geometry(shape):
+    """(n_rays, n_cells) of a per-cell array shape: [n] is n uniform slabs, [n_rays, n_cells] rays."""
+    if len(shape) <= 1:
+        return (int(np.prod(shape)) if shape else 1), 1
+    if len(shape) == 2:
+        return int(shape[0]), int(shape[1])
+    raise ValueError(f"per-cell arrays are [n] (slabs) or [n_rays, n_cells], got shape {shape}")
+
+
+def _per_cell(x, shape):
+    return np.ascontiguousarray(np.broadcast_to(np.asarray(x, dtype=np.float64), shape)).reshape(-1)
+
+
+def transfer(coeffs_cgs, psi, ds, stokes0=None, *, device=-1):
+    """Emergent Stokes ``(I, Q, U, V)`` of rays of cells with constant coefficients.
+
+    ``coeffs_cgs`` is ``[8, n]`` (n uniform slabs) or ``[8, n_rays, n_cells]``, in the order of
+    ``COEFFICIENT_NAMES`` and the units of ``compute_all_cgs``; cell 0 is where a ray enters.
+    ``psi`` (radian) and ``ds`` (cm) broadcast to the cell shape; ``stokes0`` (incident, ``[4]`` or
+    ``[4, n_rays]``) defaults to zero.  Returns ``(stokes [4, n_rays], status [n_rays])``; a ray
+    with a non-finite input, a negative length or a cell out of range (``alpha_I ds`` below -10, or
+    ``alpha_I ds``, ``|alpha_pol| ds``, ``|rho| ds`` above 1e102) is NaN with ``STATUS_NAN``.
+    """
+    c = np.asarray(coeffs_cgs, dtype=np.float64)
+    if c.ndim not in (2, 3) or c.shape[0] != 8:
+        raise ValueError(f"coeffs_cgs must be [8, n] or [8, n_rays, n_cells], got shape {c.shape}")
+    cell_shape = c.shape[1:]
+    n_rays, n_cells = _ray_geometry(cell_shape)
+    c = np.ascontiguousarray(c).reshape(8, -1)
+    psi, ds = _per_cell(psi, cell_shape), _per_cell(ds, cell_shape)
+    s0 = None if stokes0 is None else np.ascontiguousarray(
+        np.broadcast_to(np.asarray(stokes0, dtype=np.float64).reshape(4, -1), (4, n_rays)))
+    out = np.empty((4, n_rays))
+    status = np.zeros(n_rays, dtype=np.int32)
+    dp = lambda a: a.ctypes.data_as(_lib.c_double_p)  # noqa: E731
+    L = _lib.load()
+    with _lib.current_device(device):
+        rc = L.rimphony_b200_transfer(n_rays, n_cells, dp(c), dp(psi), dp(ds), dp(s0) if s0 is not None else None,
+                                      dp(out), status.ctypes.data_as(_lib.c_int32_p))
+    _lib.check(rc)
+    return out, status
+
+
+def transfer_device(coeffs8, psi, ds, stokes4, stokes0=None, status=None, *, stream=None, synchronize=True):
+    """Device-resident ``transfer``: CUDA ``torch.Tensor`` arguments (float64, contiguous; ``status``
+    int32) on one device, nothing copied.  ``coeffs8`` holds ``8 n`` values, ``psi`` and ``ds`` ``n``,
+    ``stokes4`` (and ``stokes0``) ``4 n_rays``; ``n_cells = n / n_rays``.  ``stream`` is a
+    ``torch.cuda.Stream`` (default: the library's own); with ``synchronize=False`` the call returns
+    once the kernel is enqueued."""
+    import torch
+
+    n_rays = stokes4.numel() // 4
+    n = psi.numel()
+    for t in (coeffs8, psi, ds, stokes4) + ((stokes0,) if stokes0 is not None else ()):
+        if not (t.is_cuda and t.dtype == torch.float64 and t.is_contiguous()):
+            raise ValueError("device path needs contiguous float64 CUDA tensors")
+    if status is not None and not (status.is_cuda and status.dtype == torch.int32 and status.is_contiguous()):
+        raise ValueError("status must be a contiguous int32 CUDA tensor")
+    tensors = (coeffs8, psi, ds, stokes4) + tuple(t for t in (stokes0, status) if t is not None)
+    if any(t.device != stokes4.device for t in tensors):
+        raise ValueError("all tensors must be on the device of stokes4")
+    if status is not None and status.numel() != n_rays:
+        raise ValueError("status must have n_rays values")
+    if stokes4.numel() != 4 * n_rays or n_rays == 0 or n % n_rays or coeffs8.numel() != 8 * n or ds.numel() != n:
+        raise ValueError("need coeffs8 of 8 n, psi and ds of n and stokes4 of 4 n_rays values, n_rays dividing n")
+    if stokes0 is not None and stokes0.numel() != 4 * n_rays:
+        raise ValueError("stokes0 must have 4 n_rays values")
+    L = _lib.load()
+    with _lib.current_device(stokes4.device.index):
+        rc = L.rimphony_b200_transfer_device(
+            n_rays, n // n_rays, coeffs8.data_ptr(), psi.data_ptr(), ds.data_ptr(),
+            stokes0.data_ptr() if stokes0 is not None else None, stokes4.data_ptr(),
+            status.data_ptr() if status is not None else None,
+            stream.cuda_stream if stream is not None else None, 1 if synchronize else 0)
+    _lib.check(rc)
+
+
+class StokesResult:
+    """What ``compute_stokes_cgs`` returns: ``stokes`` ``[4, n_rays]`` (I, Q, U, V), ``status``
+    ``[n_rays]`` (the OR of the cells' status words, ``STATUS_NAN`` if the ray is NaN) and ``coeffs``,
+    the cells' cgs coefficients, ``[8, n_rays, n_cells]``."""
+
+    def __init__(self, stokes, status, coeffs):
+        self.stokes = stokes
+        self.status = status
+        self.coeffs = coeffs
+
+
+def compute_stokes_cgs(kind, nu, b, n_e, theta, psi, ds, params, *, mode=MODE_FAST, device=-1, **tolerances):
+    """Coefficients and transfer in one call on the device (``rimphony_b200_compute_stokes_cgs``).
+    The per-cell arguments and the distribution's parameter columns broadcast together to ``[n]``
+    (n uniform slabs) or ``[n_rays, n_cells]``; rays enter with no radiation.  Returns a
+    ``StokesResult``."""
+    shape = np.broadcast_shapes(*(np.shape(x) for x in (nu, b, n_e, theta, psi, ds)),
+                                *(np.shape(p) for p in params))
+    n_rays, n_cells = _ray_geometry(shape)
+    cols = [_per_cell(x, shape) for x in (nu, b, n_e, theta, psi, ds)]
+    pcols, bmask = [], 0
+    for j, p in enumerate(params):
+        if np.ndim(p) == 0:
+            pcols.append(np.full(1, float(p)))
+            bmask |= 1 << j
+        else:
+            pcols.append(_per_cell(p, shape))
+    dp = lambda a: a.ctypes.data_as(_lib.c_double_p)  # noqa: E731
+    ptrs = (_lib.c_double_p * max(len(pcols), 1))(*[dp(c) for c in pcols])
+    opts = make_options(mode=mode, broadcast_mask=bmask, device=device, **tolerances)
+    stokes = np.empty((4, n_rays))
+    coeffs = np.empty((8, n_rays * n_cells))
+    status = np.zeros(n_rays, dtype=np.int32)
+    rc = _lib.load().rimphony_b200_compute_stokes_cgs(
+        kind, n_rays, n_cells, *[dp(c) for c in cols], ptrs, len(pcols), ctypes.byref(opts), dp(stokes), dp(coeffs),
+        status.ctypes.data_as(_lib.c_int32_p))
+    _lib.check(rc)
+    return StokesResult(stokes, status, coeffs.reshape(8, n_rays, n_cells))
+
+
+# ---------------------------------------------------------------------------
 # The reference's calculator trait and distribution types.
 
 
@@ -329,6 +455,15 @@ class FullSynchrotronCalculator(SynchrotronCalculator):
     def compute_all_dimensionless_batch(self, s, theta, extras=False):
         """The additive batch entry point (SURVEY.md section 8-b): returns a ``BatchResult``."""
         return self._batch(np.atleast_1d(np.asarray(s, dtype=np.float64)), theta, 0xFF, extras=extras)
+
+    def compute_stokes_cgs(self, nu, b, n_e, theta, psi, ds):
+        """Emergent Stokes ``(I, Q, U, V)`` of uniform slabs (arguments of shape ``[n]`` or scalars) or
+        of rays of cells (``[n_rays, n_cells]``, cell 0 where the ray enters) of this distribution:
+        the coefficients of ``compute_all_cgs`` in every cell, then ``transfer`` through the cells of
+        length ``ds`` (cm) with field angle ``psi``, in one call on the device.  Returns a
+        ``StokesResult``; ``.stokes`` is ``[4, n_rays]``."""
+        return compute_stokes_cgs(self.distrib.KIND, nu, b, n_e, theta, psi, ds, self.distrib._columns(),
+                                  mode=self.mode, device=self.device)
 
 
     # -- diagnostics of the Symphony double integral (src/lib.rs:249-299) ----------------

@@ -51,6 +51,9 @@ EXPORTED_SYMBOLS = (
     "rimphony_b200_diagnostic_symphony",
     "rimphony_b200_bessel_jn",
     "rimphony_b200_dist_eval",
+    "rimphony_b200_transfer",
+    "rimphony_b200_transfer_device",
+    "rimphony_b200_compute_stokes_cgs",
     "rimphony_b200_last_kernel_ms",
     "rimphony_b200_fp64_peak_tflops",
     "rimphony_b200_kernel_launch_count",
@@ -90,6 +93,11 @@ def load():
                                                     c_double_p, c_double_p, c_int32_p]
     L.rimphony_b200_bessel_jn.argtypes = [i64, c_double_p, c_double_p, c_double_p, c_double_p]
     L.rimphony_b200_dist_eval.argtypes = [i32, c_double_p, i32, i64, c_double_p, c_double_p, c_double_p]
+    L.rimphony_b200_transfer.argtypes = [i64, i64, c_double_p, c_double_p, c_double_p, c_double_p, c_double_p, c_int32_p]
+    L.rimphony_b200_transfer_device.argtypes = [i64, i64, vp, vp, vp, vp, vp, vp, vp, i32]
+    L.rimphony_b200_compute_stokes_cgs.argtypes = [i32, i64, i64, c_double_p, c_double_p, c_double_p, c_double_p,
+                                                   c_double_p, c_double_p, pp, i32, OP, c_double_p, c_double_p,
+                                                   c_int32_p]
     L.rimphony_b200_last_kernel_ms.argtypes = [i32, ctypes.POINTER(ctypes.c_float)]
     L.rimphony_b200_fp64_peak_tflops.argtypes = [i32, c_double_p]
     L.rimphony_b200_kernel_launch_count.restype = ctypes.c_uint64
@@ -97,6 +105,27 @@ def load():
     L.rimphony_b200_shutdown.restype = None
     _lib = L
     return L
+
+
+class current_device:
+    """Within the block, the calling thread's current CUDA device (of the CUDA runtime the library uses) is
+    `device`; -1 leaves it as it is.  The entry points without an options struct run there."""
+
+    def __init__(self, device):
+        self.device, self.saved = int(device), None
+
+    def __enter__(self):
+        if self.device >= 0:
+            L, cur = load(), ctypes.c_int(-1)
+            if L.cudaGetDevice(ctypes.byref(cur)) != 0 or L.cudaSetDevice(self.device) != 0:
+                raise RimphonyB200Error(f"cannot select CUDA device {self.device}")
+            self.saved = cur.value
+        return self
+
+    def __exit__(self, *exc):
+        if self.saved is not None:
+            load().cudaSetDevice(self.saved)
+        return False
 
 
 def check(rc):

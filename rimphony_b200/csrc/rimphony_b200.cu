@@ -11,6 +11,9 @@
 // 10x, so each warp of the persistent kernels pulls the next point from a global atomic counter.
 // All arithmetic is FP64 on the CUDA cores; there is no dense contraction for the tensor cores to do.
 //
+// rimphony_b200_transfer* and rimphony_b200_compute_stokes_cgs add the polarized transfer through rays of cells
+// (rb_transfer.cuh, kernels in inst_transfer.cu): one thread per ray.
+//
 // There is deliberately no host implementation behind these entry points: with
 // no usable CUDA device every call fails with a nonzero return code.
 #include <cuda_runtime.h>
@@ -27,6 +30,7 @@
 
 #include "../../include/rimphony_b200.h"
 #include "rb_launch.cuh"
+#include "rb_transfer.cuh"
 
 namespace {
 
@@ -565,6 +569,27 @@ int run_host(int kind, int64_t n, const double *s, const double *theta, const do
     return collect_times(c);
 }
 
+// The argument checks of the transfer entry points; *n_points = n_rays * n_cells.
+int check_rays(int64_t n_rays, int64_t n_cells, int64_t *n_points)
+{
+    if (n_rays < 0 || n_cells < 0)
+        return fail("n_rays and n_cells must not be negative");
+    if (n_cells > 0 && n_rays > INT64_MAX / n_cells)
+        return fail("n_rays * n_cells overflows");
+    *n_points = n_rays * n_cells;
+    return 0;
+}
+
+int check_transfer(int64_t n_rays, int64_t n_cells, const double *coeffs8, const double *psi, const double *ds,
+                   const double *stokes4, int64_t *n_points)
+{
+    if (check_rays(n_rays, n_cells, n_points))
+        return 1;
+    if (n_rays > 0 && (!stokes4 || (*n_points > 0 && (!coeffs8 || !psi || !ds))))
+        return fail("null array pointer");
+    return 0;
+}
+
 } // namespace
 
 // ---------------------------------------------------------------------------
@@ -882,6 +907,155 @@ int rimphony_b200_fp64_peak_tflops(int device, double *out_tflops)
     }
     *out_tflops = best;
     return 0;
+}
+
+int rimphony_b200_transfer(int64_t n_rays, int64_t n_cells, const double *coeffs8, const double *psi, const double *ds,
+                           const double *stokes0, double *stokes4, int32_t *status)
+{
+    int64_t n;
+    if (check_transfer(n_rays, n_cells, coeffs8, psi, ds, stokes4, &n))
+        return 1;
+    if (n_rays == 0)
+        return 0;
+    DeviceGuard restore_device;
+    DeviceContext *cp = nullptr;
+    if (get_context(-1, &cp))
+        return 1;
+    DeviceContext &c = *cp;
+    std::lock_guard<std::mutex> guard(c.lock);
+    RB_CUDA(cudaSetDevice(c.device));
+
+    // device staging: [coeffs8 | psi | ds | stokes0] in, [stokes4 | status] out
+    const size_t nb = (size_t)n * sizeof(double), rb4 = 4 * (size_t)n_rays * sizeof(double);
+    if (c.in.reserve(10 * nb + rb4) || c.out.reserve(rb4 + (size_t)n_rays * sizeof(int32_t)))
+        return 1;
+    double *d_coeffs = static_cast<double *>(c.in.ptr), *d_psi = d_coeffs + 8 * n, *d_ds = d_psi + n;
+    double *d_s0 = stokes0 ? d_ds + n : nullptr;
+    double *d_stokes = static_cast<double *>(c.out.ptr);
+    int32_t *d_status = reinterpret_cast<int32_t *>(d_stokes + 4 * n_rays);
+    if (n > 0) {
+        RB_CUDA(cudaMemcpyAsync(d_coeffs, coeffs8, 8 * nb, cudaMemcpyHostToDevice, c.stream));
+        RB_CUDA(cudaMemcpyAsync(d_psi, psi, nb, cudaMemcpyHostToDevice, c.stream));
+        RB_CUDA(cudaMemcpyAsync(d_ds, ds, nb, cudaMemcpyHostToDevice, c.stream));
+    }
+    if (stokes0)
+        RB_CUDA(cudaMemcpyAsync(d_s0, stokes0, rb4, cudaMemcpyHostToDevice, c.stream));
+    RB_CUDA(launch_transfer(n_rays, n_cells, d_coeffs, d_psi, d_ds, d_s0, nullptr, d_stokes, d_status, c.stream));
+    g_launches++;
+    RB_CUDA(cudaMemcpyAsync(stokes4, d_stokes, rb4, cudaMemcpyDeviceToHost, c.stream));
+    if (status)
+        RB_CUDA(cudaMemcpyAsync(status, d_status, (size_t)n_rays * sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
+    RB_CUDA(cudaStreamSynchronize(c.stream));
+    return 0;
+}
+
+int rimphony_b200_transfer_device(int64_t n_rays, int64_t n_cells, const double *coeffs8, const double *psi,
+                                  const double *ds, const double *stokes0, double *stokes4, int32_t *status,
+                                  void *stream, int synchronize)
+{
+    int64_t n;
+    if (check_transfer(n_rays, n_cells, coeffs8, psi, ds, stokes4, &n))
+        return 1;
+    if (n_rays == 0)
+        return 0;
+    DeviceGuard restore_device;
+    DeviceContext *cp = nullptr;
+    if (get_context(-1, &cp))
+        return 1;
+    DeviceContext &c = *cp;
+    std::lock_guard<std::mutex> guard(c.lock);
+    RB_CUDA(cudaSetDevice(c.device));
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : c.stream;
+    RB_CUDA(launch_transfer(n_rays, n_cells, coeffs8, psi, ds, stokes0, nullptr, stokes4, status, st));
+    g_launches++;
+    if (synchronize)
+        RB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+int rimphony_b200_compute_stokes_cgs(int kind, int64_t n_rays, int64_t n_cells, const double *nu, const double *b,
+                                     const double *n_e, const double *theta, const double *psi, const double *ds,
+                                     const double *const *params, int n_params, const rimphony_b200_options *opts,
+                                     double *stokes4, double *coeffs8_cgs, int32_t *status)
+{
+    int64_t n;
+    if (check_rays(n_rays, n_cells, &n))
+        return 1;
+    ResolvedOptions o;
+    if (check_batch(kind, n, nu, theta, params, n_params, stokes4, opts, &o))
+        return 1;
+    if (n_rays == 0)
+        return 0;
+    if (!stokes4)
+        return fail("null array pointer");
+    if (n == 0) { // rays without cells: nothing enters, nothing is emitted
+        for (int64_t i = 0; i < 4 * n_rays; i++)
+            stokes4[i] = 0.0;
+        if (status)
+            memset(status, 0, (size_t)n_rays * sizeof(int32_t));
+        return 0;
+    }
+    if (!b || !n_e || !psi || !ds)
+        return fail("null array pointer");
+    if (o.coeff_mask != 0xFFu)
+        return fail("compute_stokes_cgs needs all eight coefficients: coeff_mask must be 0 or 0xFF, got 0x%x",
+                    o.coeff_mask);
+    for (int j = 0; j < n_params; j++)
+        if (!params[j])
+            return fail("params[%d] is null", j);
+    DeviceGuard restore_device;
+    DeviceContext *cp = nullptr;
+    if (get_context(o.device, &cp))
+        return 1;
+    DeviceContext &c = *cp;
+    std::lock_guard<std::mutex> guard(c.lock);
+    RB_CUDA(cudaSetDevice(c.device));
+
+    // device staging: [nu | b | n_e | theta | psi | ds | s | param columns] in,
+    // [out8 | norm | stokes4 | cell status | ray status] out
+    const size_t nb = (size_t)n * sizeof(double);
+    size_t in_doubles = 7 * (size_t)n;
+    for (int j = 0; j < n_params; j++)
+        in_doubles += ((o.bcast >> j) & 1u) ? 1 : (size_t)n;
+    const size_t out_bytes = 9 * nb + 4 * (size_t)n_rays * sizeof(double) + (size_t)(n + n_rays) * sizeof(int32_t);
+    if (c.in.reserve(in_doubles * sizeof(double)) || c.out.reserve(out_bytes))
+        return 1;
+    double *d_nu = static_cast<double *>(c.in.ptr), *d_b = d_nu + n, *d_ne = d_b + n, *d_theta = d_ne + n;
+    double *d_psi = d_theta + n, *d_ds = d_psi + n, *d_s = d_ds + n;
+    const double *host_cols[6] = {nu, b, n_e, theta, psi, ds};
+    for (int k = 0; k < 6; k++)
+        RB_CUDA(cudaMemcpyAsync(d_nu + k * n, host_cols[k], nb, cudaMemcpyHostToDevice, c.stream));
+    const double *d_params[kMaxParams] = {};
+    double *cur = d_s + n;
+    for (int j = 0; j < n_params; j++) {
+        const size_t cnt = ((o.bcast >> j) & 1u) ? 1 : (size_t)n;
+        RB_CUDA(cudaMemcpyAsync(cur, params[j], cnt * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+        d_params[j] = cur;
+        cur += cnt;
+    }
+    double *d_out8 = static_cast<double *>(c.out.ptr), *d_norm = d_out8 + 8 * n, *d_stokes = d_norm + n;
+    int32_t *d_cell_status = reinterpret_cast<int32_t *>(d_stokes + 4 * n_rays), *d_status = d_cell_status + n;
+
+    RB_CUDA(launch_cgs_s(n, d_nu, d_b, d_s, c.stream));
+    g_launches++;
+    rimphony_b200_extras dev_extras;
+    dev_extras.lobes4 = nullptr;
+    dev_extras.counters = nullptr;
+    dev_extras.norm = d_norm;
+    if (run_device(kind, n, d_s, d_theta, d_params, n_params, o, d_out8, d_cell_status, &dev_extras, nullptr, 0, c))
+        return 1;
+    RB_CUDA(launch_cgs_scale(n, d_nu, d_ne, d_out8, c.stream));
+    g_launches++;
+    RB_CUDA(launch_transfer(n_rays, n_cells, d_out8, d_psi, d_ds, nullptr, d_cell_status, d_stokes, d_status, c.stream));
+    g_launches++;
+
+    RB_CUDA(cudaMemcpyAsync(stokes4, d_stokes, 4 * (size_t)n_rays * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
+    if (coeffs8_cgs)
+        RB_CUDA(cudaMemcpyAsync(coeffs8_cgs, d_out8, 8 * nb, cudaMemcpyDeviceToHost, c.stream));
+    if (status)
+        RB_CUDA(cudaMemcpyAsync(status, d_status, (size_t)n_rays * sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
+    RB_CUDA(cudaStreamSynchronize(c.stream));
+    return collect_times(c);
 }
 
 uint64_t rimphony_b200_kernel_launch_count(void) { return g_launches.load(); }

@@ -1,13 +1,16 @@
 """The reference's one-shot example programs on the GPU path.
 
     python -m rimphony_b200.examples all-pitchykappa-cgs NU B N_E THETA KAPPA WIDTH K
+    python -m rimphony_b200.examples stokes-slab-pitchykappa-cgs NU B N_E THETA PSI DEPTH KAPPA WIDTH K
     python -m rimphony_b200.examples one-powerlaw-direct
     python -m rimphony_b200.examples one-powerlaw-normalized
     python -m rimphony_b200.examples one-pitchypl-normalized
 
 Same positional arguments, constants and output lines as ``examples/all-pitchykappa-cgs.rs:13-133``,
 ``one-powerlaw-direct.rs:10-30``, ``one-powerlaw-normalized.rs:13-47`` and
-``one-pitchypl-normalized.rs:11-29``.  (The crank-out tools and ``demo-powerlaw`` are in
+``one-pitchypl-normalized.rs:11-29``.  ``stokes-slab-pitchykappa-cgs`` has no counterpart in the
+reference: it prints the emergent Stokes I, Q, U, V of a uniform slab of depth DEPTH (cm) with the
+coefficients ``all-pitchykappa-cgs`` prints and field angle PSI.  (The crank-out tools and ``demo-powerlaw`` are in
 ``rimphony_b200.crank_out``.)  ``--mode faithful`` runs the reference's own sequence of rule
 applications instead of the product path.
 """
@@ -55,6 +58,16 @@ def all_pitchykappa_cgs(args, R, out):
     return 0
 
 
+def stokes_slab_pitchykappa_cgs(args, R, out):
+    """Emergent (I, Q, U, V) of a uniform slab of the all-pitchykappa-cgs distribution (gamma cutoff 100)."""
+    calc = (R.PitchyKappaDistribution(args.KAPPA, args.WIDTH, args.K).gamma_cutoff(100.0)
+            .full_calculation(mode=args.mode))
+    res = calc.compute_stokes_cgs(args.NU, args.B, args.N_E, args.THETA, args.PSI, args.DEPTH)
+    for label, v in zip(("I", "Q", "U", "V"), res.stokes[:, 0]):
+        out.write(f"{label}: {rust_e(float(v), 18)}\n")
+    return 0
+
+
 def one_powerlaw_direct(args, R, out):
     """examples/one-powerlaw-direct.rs:10-30."""
     symphony_ji = 2.64399749412774e-21
@@ -88,7 +101,8 @@ def one_pitchypl_normalized(args, R, out):
     return 0
 
 
-TOOLS = {"all-pitchykappa-cgs": all_pitchykappa_cgs, "one-powerlaw-direct": one_powerlaw_direct,
+TOOLS = {"all-pitchykappa-cgs": all_pitchykappa_cgs, "stokes-slab-pitchykappa-cgs": stokes_slab_pitchykappa_cgs,
+         "one-powerlaw-direct": one_powerlaw_direct,
          "one-powerlaw-normalized": one_powerlaw_normalized, "one-pitchypl-normalized": one_pitchypl_normalized}
 
 
@@ -100,6 +114,9 @@ def parse(argv):
     cgs = sub.add_parser("all-pitchykappa-cgs")
     for name in ("NU", "B", "N_E", "THETA", "KAPPA", "WIDTH", "K"):
         cgs.add_argument(name, type=float)
+    slab = sub.add_parser("stokes-slab-pitchykappa-cgs")
+    for name in ("NU", "B", "N_E", "THETA", "PSI", "DEPTH", "KAPPA", "WIDTH", "K"):
+        slab.add_argument(name, type=float)
     for name in ("one-powerlaw-direct", "one-powerlaw-normalized", "one-pitchypl-normalized"):
         sub.add_parser(name)
     return ap.parse_args(argv)

@@ -53,6 +53,18 @@ extern "C" {
                                    dj: *mut c_double) -> c_int;
     pub fn rimphony_b200_dist_eval(kind: c_int, params: *const c_double, n_params: c_int, count: i64,
                                    gamma: *const c_double, cos_xi: *const c_double, out3: *mut c_double) -> c_int;
+    pub fn rimphony_b200_transfer(
+        n_rays: i64, n_cells: i64, coeffs8: *const c_double, psi: *const c_double, ds: *const c_double,
+        stokes0: *const c_double, stokes4: *mut c_double, status: *mut i32) -> c_int;
+    pub fn rimphony_b200_transfer_device(
+        n_rays: i64, n_cells: i64, coeffs8: *const c_double, psi: *const c_double, ds: *const c_double,
+        stokes0: *const c_double, stokes4: *mut c_double, status: *mut i32, stream: *mut c_void,
+        synchronize: c_int) -> c_int;
+    pub fn rimphony_b200_compute_stokes_cgs(
+        kind: c_int, n_rays: i64, n_cells: i64, nu: *const c_double, b: *const c_double, n_e: *const c_double,
+        theta: *const c_double, psi: *const c_double, ds: *const c_double, params: *const *const c_double,
+        n_params: c_int, opts: *const Options, stokes4: *mut c_double, coeffs8_cgs: *mut c_double,
+        status: *mut i32) -> c_int;
     pub fn rimphony_b200_last_kernel_ms(device: c_int, out_ms: *mut c_float) -> c_int;
     pub fn rimphony_b200_fp64_peak_tflops(device: c_int, out_tflops: *mut c_double) -> c_int;
     pub fn rimphony_b200_kernel_launch_count() -> u64;

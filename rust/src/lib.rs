@@ -259,6 +259,46 @@ impl<D: B200Params> FullSynchrotronCalculator<D> {
     }
 }
 
+impl<D: B200Params> FullSynchrotronCalculator<D> {
+    /// Emergent Stokes `[I, Q, U, V]` of `n_rays` rays of `n_cells` cells each of this distribution
+    /// (`rimphony_b200_compute_stokes_cgs`): the coefficients of `compute_all_cgs` in every cell, then
+    /// `transfer` with no incident radiation, in one call on the device.  `nu`, `b`, `n_e`, `theta`,
+    /// `psi` and `ds` hold one value per cell, index `ray * n_cells + cell` (cell 0 where the ray
+    /// enters); `n_cells = 1` is a set of uniform slabs.
+    pub fn compute_stokes_cgs(&self, n_cells: usize, nu: &[f64], b: &[f64], n_e: &[f64], theta: &[f64],
+                              psi: &[f64], ds: &[f64]) -> Result<TransferResult, String>
+    {
+        let n = nu.len();
+        if n_cells == 0 || n % n_cells != 0 {
+            return Err(format!("{} cells do not make rays of {} cells", n, n_cells));
+        }
+        if [b.len(), n_e.len(), theta.len(), psi.len(), ds.len()].iter().any(|&l| l != n) {
+            return Err("nu, b, n_e, theta, psi and ds differ in length".into());
+        }
+        let n_rays = n / n_cells;
+        let p = self.distrib.b200_params();
+        let ptrs: Vec<*const c_double> = p.iter().map(|v| v as *const f64).collect();
+        let opts = ffi::Options {
+            struct_size: std::mem::size_of::<ffi::Options>() as u32,
+            mode: self.mode as i32,
+            param_broadcast_mask: (1u32 << p.len()) - 1,
+            ..Default::default()
+        };
+        let mut soa = vec![f64::NAN; 4 * n_rays];
+        let mut status = vec![0i32; n_rays];
+        let rc = unsafe {
+            ffi::rimphony_b200_compute_stokes_cgs(D::KIND, n_rays as i64, n_cells as i64, nu.as_ptr(), b.as_ptr(),
+                                                  n_e.as_ptr(), theta.as_ptr(), psi.as_ptr(), ds.as_ptr(),
+                                                  ptrs.as_ptr(), ptrs.len() as c_int, &opts, soa.as_mut_ptr(),
+                                                  std::ptr::null_mut(), status.as_mut_ptr())
+        };
+        if rc != 0 {
+            return Err(last_error());
+        }
+        Ok(TransferResult::from_soa(&soa, status))
+    }
+}
+
 impl<D: B200Params> SynchrotronCalculator for FullSynchrotronCalculator<D> {
     fn compute_dimensionless(&self, coeff: Coefficient, stokes: Stokes, s: f64, theta: f64) -> f64 {
         let p = self.distrib.b200_params();
@@ -344,6 +384,58 @@ pub fn compute_all_dimensionless_multi(kind: c_int, s: &[f64], theta: &[f64], co
     }
     let values = (0..n).map(|i| { let mut r = [0.0; 8]; for c in 0..8 { r[c] = soa[c * n + i]; } r }).collect();
     Ok(BatchResult { values, status })
+}
+
+/// Emergent Stokes vectors of a set of rays: `stokes[ray] = [I, Q, U, V]`, and the per-ray status
+/// word (`status::NAN` if the ray's vector is NaN).
+pub struct TransferResult {
+    pub stokes: Vec<[f64; 4]>,
+    pub status: Vec<i32>,
+}
+
+impl TransferResult {
+    fn from_soa(soa: &[f64], status: Vec<i32>) -> Self {
+        let n = status.len();
+        let stokes = (0..n).map(|r| [soa[r], soa[n + r], soa[2 * n + r], soa[3 * n + r]]).collect();
+        TransferResult { stokes, status }
+    }
+}
+
+/// Polarized transfer through rays of cells with constant coefficients (`rimphony_b200_transfer`; the
+/// matrix and its sign convention are in include/rimphony_b200.h).  `coeffs[p]` is the cgs vector of
+/// `compute_all_cgs` of cell `p = ray * n_cells + cell`, cell 0 where the ray enters; `psi` and `ds`
+/// hold one value per cell; `stokes0` is the incident `[I, Q, U, V]` of each ray (zero if `None`).
+pub fn transfer(n_cells: usize, coeffs: &[[f64; 8]], psi: &[f64], ds: &[f64], stokes0: Option<&[[f64; 4]]>)
+    -> Result<TransferResult, String>
+{
+    let n = coeffs.len();
+    if n_cells == 0 || n % n_cells != 0 || psi.len() != n || ds.len() != n {
+        return Err(format!("{} cells with {} angles and {} lengths do not make rays of {} cells",
+                           n, psi.len(), ds.len(), n_cells));
+    }
+    let n_rays = n / n_cells;
+    let mut soa = vec![0.0; 8 * n];
+    for (p, c) in coeffs.iter().enumerate() {
+        for k in 0..8 {
+            soa[k * n + p] = c[k];
+        }
+    }
+    let s0: Option<Vec<f64>> = match stokes0 {
+        Some(v) if v.len() != n_rays => return Err("stokes0 needs one vector per ray".into()),
+        Some(v) => Some((0..4 * n_rays).map(|i| v[i % n_rays][i / n_rays]).collect()),
+        None => None,
+    };
+    let mut out = vec![f64::NAN; 4 * n_rays];
+    let mut status = vec![0i32; n_rays];
+    let rc = unsafe {
+        ffi::rimphony_b200_transfer(n_rays as i64, n_cells as i64, soa.as_ptr(), psi.as_ptr(), ds.as_ptr(),
+                                    s0.as_ref().map_or(std::ptr::null(), |v| v.as_ptr()), out.as_mut_ptr(),
+                                    status.as_mut_ptr())
+    };
+    if rc != 0 {
+        return Err(last_error());
+    }
+    Ok(TransferResult::from_soa(&out, status))
 }
 
 /// leung-bessel/src/lib.rs:56-75 on the device: `(J_n(x), J_n'(x))` for arrays of arguments.
